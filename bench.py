@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle) on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed as DIR/*.npy
 
 metric   : input bytes/sec of DFA witness generation (state column, substr ids, enable bitmaps, masked chars/ids,
            status, records, lookup multiplicities) — bit-exact outputs, see tests/.
@@ -251,6 +252,54 @@ def oracle_tile_check(H, cfg, ocfg, d_bytes, L, out, lo, cnt=256):
     return not errs
 
 
+DUMP_STRINGS = 1024        # strings in the --dump-outputs sample: ~25 MB as float32 for config 1
+DUMP_SEED = 0xB200D0       # the sample is the same strings in every run
+
+
+def dump_outputs(out, directory):
+    """--dump-outputs: the witness of the timed path's last step as DIR/<name>.npy (float32, counters float64) — every column
+    of a fixed, seeded sample of the batch's strings, restricted to what include/b2r.h defines (rows [0, M), the first
+    n_records records, the first n_compact compacted bytes; the rest of each buffer is left unspecified and zeroed here), and
+    every multiplicity counter of the batch."""
+    import numpy as np
+    import torch
+    from b2r_layout import abi as _abi
+    os.makedirs(directory, exist_ok=True)
+    n, m = out.n, out.m
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_STRINGS), replace=False))
+    rows = torch.from_numpy(idx).to(out.mult_all.device)
+
+    def take(t):
+        a = t.index_select(0, rows).cpu().numpy()
+        return a.view(np.uint16) if a.dtype == np.int16 else a
+
+    def bits(t):
+        return np.unpackbits(take(t), axis=1, bitorder="little")[:, :m]
+
+    arrays = {"string_index": idx.astype(np.float64)}
+    for d in range(out.cfg.n_defs):
+        arrays[f"states{d}"] = take(out.states[d])[:, :m]
+        arrays[f"substr_ids{d}"] = take(out.substr_ids[d])[:, :m]
+        arrays[f"start_enable{d}"] = bits(out.start_enable[d])
+        arrays[f"end_enable{d}"] = bits(out.end_enable[d])
+        arrays[f"mult{d}"] = out.mult[d].cpu().numpy().astype(np.float64)
+        arrays[f"endpoint_mult{d}"] = out.endpoint_mult[d].cpu().numpy().astype(np.float64)
+    arrays["masked_chars"] = take(out.masked_chars)[:, :m]
+    arrays["masked_substr_ids"] = take(out.masked_substr_ids)[:, :m]
+    status = take(out.status).reshape(-1).view(_abi.STATUS_DTYPE)
+    for f in ("flags", "err_pos", "err_state", "err_byte", "err_def", "n_records", "n_compact"):
+        arrays["status_" + f] = status[f].astype(np.float64)
+    records = take(out.records).view(_abi.RECORD_DTYPE).reshape(len(idx), out.max_records)
+    records = np.stack([records[f] for f, _ in _abi.RECORD_DTYPE], axis=-1).astype(np.float64)
+    records[np.arange(out.max_records)[None, :] >= status["n_records"][:, None]] = 0
+    arrays["records"] = records
+    compact = take(out.compact_bytes).astype(np.float32)
+    compact[np.arange(out.compact_pitch)[None, :] >= status["n_compact"][:, None]] = 0
+    arrays["compact_bytes"] = compact
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
+
+
 def gathered_mult_check(ctx, local, reduced):
     """N > 1: the all-reduced counters against the host sum of the all-gathered per-rank counters, row by row."""
     if ctx.world == 1:
@@ -262,8 +311,9 @@ def gathered_mult_check(ctx, local, reduced):
     return bool((host_sum == reduced.cpu().numpy().astype("uint64")).all())
 
 
-def batch_leg(ctx, H, W, key, workload, cfg, ocfg, d_bytes, n, L, m, steps, warmup, max_records=2, compact_pitch=8):
-    """One batch config with the inputs resident in HBM: device-timed steps, the kernel alone, parity checks."""
+def batch_leg(ctx, H, W, key, workload, cfg, ocfg, d_bytes, n, L, m, steps, warmup, max_records=2, compact_pitch=8, dump_dir=None):
+    """One batch config with the inputs resident in HBM: device-timed steps, the kernel alone, parity checks; `dump_dir`: where
+    dump_outputs() writes what the last timed step computed."""
     import numpy as np
     torch, world, rank, dev = ctx.torch, ctx.world, ctx.rank, ctx.dev
     from halo2_regex_b200 import _abi
@@ -315,6 +365,8 @@ def batch_leg(ctx, H, W, key, workload, cfg, ocfg, d_bytes, n, L, m, steps, warm
         torch.cuda.profiler.stop()
     clocks = sampler.stop() if sampler else None
     assert cfg.batch_result(stream=ctx.stream()).code == 0
+    if dump_dir:
+        dump_outputs(out, dump_dir)
 
     # ---- parity, outside the timed region -------------------------------------------------------------------------------------
     reduced = out.mult_all.clone()
@@ -538,7 +590,7 @@ def latency_leg(ctx, H, cfg, ocfg):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline config (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--log2-strings", type=int, default=LOG2_STRINGS, help="strings per GPU (default: the BASELINE config)")
@@ -551,7 +603,13 @@ def main():
     ap.add_argument("--log2-long", type=int, default=26, help="config 3: log2 of the string length")
     ap.add_argument("--no-long-oracle", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the single-process multi-device leg and the one-string latency leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the headline config's last step computed "
+                    "(a fixed sample of its strings, every multiplicity counter) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; the reference arm has none")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return reference_arm(args)
@@ -571,7 +629,8 @@ def main():
     cfg = make_config(H, SET_REGEX1, M, ctx.local_rank)
     ocfg1 = oracle_from_files(SET_REGEX1, M)
     d_bytes = W.config1_torch(n, L, first=rank * n, device=dev).reshape(-1)      # this rank's slice of the global batch
-    head, out, d_offs, clocks = batch_leg(ctx, H, W, "1", workload_config(args.log2_strings)["workload"], cfg, ocfg1, d_bytes, n, L, M, args.steps, args.warmup)
+    head, out, d_offs, clocks = batch_leg(ctx, H, W, "1", workload_config(args.log2_strings)["workload"], cfg, ocfg1, d_bytes, n, L, M, args.steps, args.warmup,
+                                          dump_dir=args.dump_outputs if rank == 0 else None)
     del out, d_offs
 
     # ---- end-to-end arm: C-ABI call with pinned host buffers -----------------------------------------------------------------------
