@@ -517,8 +517,9 @@ int b2r_match_long(b2r_config* c, const uint8_t* d_bytes, uint64_t len, const b2
     if ((rc = c->ws_long.reserve(need))) return rc;
     unsigned char* ws = (unsigned char*)c->ws_long.p;
     uint64_t* d_offsets = (uint64_t*)(ws + off_offsets);
-    // (the {0, len} pair of the whole string behind the chunk offsets is written by the kernel that writes those: no host copy on this
-    // path, so a caller may capture it in a CUDA graph)
+    // (the {0, len} pair of the whole string behind the chunk offsets is written by the kernel that writes those, and the root entry
+    // state of the composition tree by long_root_kernel: no host copy on this path, so a caller may capture it in a CUDA graph once a
+    // first call of the same length has sized the workspace)
 
     // ---- 1 + 2: transition vectors of the chunks, composition tree, entry state of every chunk ------------------------------
     LongParams lp;

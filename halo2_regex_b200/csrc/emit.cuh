@@ -538,6 +538,8 @@ struct TileEmitter {
             __syncwarp();
             if (patch) { ls.template scan<true>(fw0, fw1, p.fmask); r_nrec = ls.n_rec; r_ncmp = ls.n_cmp; }
         }
+        // two defs flagging one row: the string has no records (include/b2r.h), so no counts and no truncation flags either
+        if (r_flags & B2R_ST_OVERLAP) { r_nrec = 0; r_ncmp = 0; }
 
         // ---- accept rule (src/lib.rs:427-457), status records (lane = string) --------------------------------------------
         if (valid && !(p.debug & 8)) {

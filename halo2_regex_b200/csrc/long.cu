@@ -209,6 +209,10 @@ __global__ void __launch_bounds__(256) long_propagate_kernel(const uint16_t* chi
     for (uint32_t c = c0; c < c1; c++) { child_entry[c] = (uint16_t)s; s = child_maps[(size_t)c * S1 + s]; }
 }
 
+// the root of the composition tree starts in first_state.  Written by a kernel rather than copied from the host, so that the
+// long-string path stays capturable in a CUDA graph (a captured host copy would read this call's stack variable at every replay)
+__global__ void long_root_kernel(uint16_t* root_entry, uint32_t first) { *root_entry = (uint16_t)first; }
+
 // The same tree with one CTA per parent node: a Hillis-Steele scan (composition is associative, not commutative: earlier
 // children are applied first) over its <= 64 children in shared memory.  The child maps are replaced IN PLACE by their
 // exclusive prefixes E_c = f_{c-1} o ... o f_0 (E_0 = identity); the parent gets the composition of all of them.
@@ -629,6 +633,7 @@ __global__ void __launch_bounds__(128) long_emit_kernel(const __grid_constant__ 
         pass(std::true_type{});
         if (lane == 0) { r_nrec = ls.n_rec; r_ncmp = ls.n_cmp; }
     }
+    if (lane == 0 && (r_flags & B2R_ST_OVERLAP)) { r_nrec = 0; r_ncmp = 0; }   // no records for a string two defs flag on one row
     if (lane == 0) {
         uint32_t fin[D];
 #pragma unroll
@@ -762,8 +767,8 @@ int launch_long_prepare(const LongParams& lp, void* stream, uint32_t* launches) 
             LAUNCH_CHECK("long_compose_kernel"); (*launches)++;
         }
         // the root starts in first_state; down the tree
-        const uint16_t first = (uint16_t)lp.def[d].first_state;
-        if (cudaMemcpyAsync(lp.def[d].entry + off_level.back(), &first, 2, cudaMemcpyHostToDevice, st) != cudaSuccess) { set_error("cudaMemcpyAsync(entry)"); return B2R_ERR_CUDA; }
+        long_root_kernel<<<1, 1, 0, st>>>(lp.def[d].entry + off_level.back(), lp.def[d].first_state);
+        LAUNCH_CHECK("long_root_kernel"); (*launches)++;
         for (size_t l = n_level.size() - 1; l-- > 0;) {
             const uint32_t nc = n_level[l], np = n_level[l + 1];
             long_propagate_kernel<<<(np + 255) / 256, 256, 0, st>>>(lp.def[d].maps + off_level[l] * S1, lp.def[d].entry + off_level[l + 1], lp.def[d].entry + off_level[l], nc, np, S1);

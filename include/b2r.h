@@ -153,7 +153,8 @@ int b2r_endpoint_rows(const b2r_config*, uint32_t d, uint64_t* out3, uint64_t ca
 #define B2R_ST_ACCEPTED(d) (1u << (d))     /* state[len] == accepted_state_val of def d (src/lib.rs:427-457) */
 #define B2R_ST_OVERLAP (1u << 8)           /* two defs flagged the same row (is_start or is_end sum > 1): the reference's
                                               and/not/select arithmetic is non-boolean there (src/lib.rs:613-642);
-                                              masked outputs / records of this string are unspecified */
+                                              masked outputs of this string are unspecified, and it has no records:
+                                              n_records = n_compact = 0, no truncation flag */
 #define B2R_ST_INVALID_TRANSITION (1u << 9) /* reference panics (src/lib.rs:817); err_* describe the first one */
 #define B2R_ST_TOO_LONG (1u << 10)         /* len > max_chars_size-1 (or offsets outside the byte buffer): string skipped, its rows are unspecified */
 #define B2R_ST_RECORDS_TRUNCATED (1u << 11)

@@ -60,9 +60,10 @@ def test_golden_states_survey():
         assert int(out.states[0][0, len(text)]) == final
 
 
-def _compare_with_pyref(set_name, M, strings):
-    cfg = oracle_config(set_name, M)
-    pdefs = pyref_defs(set_name)
+def _compare_with_pyref(set_name, M, strings, cfg=None, pdefs=None):
+    """set_name: a DEF_SETS entry, or None with `cfg` (an OracleConfig) and `pdefs` (the same defs for pyref) given."""
+    cfg = cfg if cfg is not None else oracle_config(set_name, M)
+    pdefs = pdefs if pdefs is not None else pyref_defs(set_name)
     out, res = cfg.match_strings(strings, max_records=16, compact_pitch=M)
     for j, s in enumerate(strings):
         try:
