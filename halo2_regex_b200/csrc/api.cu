@@ -2,6 +2,7 @@
 // points live in host.cu.
 #include <cuda_runtime.h>
 
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <algorithm>
@@ -588,6 +589,112 @@ int b2r_match_long(b2r_config* c, const uint8_t* d_bytes, uint64_t len, const b2
     return B2R_OK;
 }
 
+// Chunked batch path: b2r_match_batch's outputs, with every string cut into K = ceil(M / LONG_CHUNK) slots that are walked in
+// parallel.  Per pass of whole strings: the slots' transition vectors (general prefix pass of long.cu), the last slot of every
+// string reset to the constant map -> first_state, the composition tree over all slots of the pass (entry state of every slot),
+// walk_kernel<..., CH = true> over the slots (state rows and flag words straight into the batch layout).  Then emit_kernel and
+// finalize_kernel over the N strings, exactly as match_batch_impl runs them when the emit stage is its own kernel.
+static int match_batch_chunked_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t total_bytes,
+                             const b2r_outputs* o, cudaStream_t st) {
+    if (c->device < 0) { set_error("this handle was created without a device (device = -1): no CPU fallback exists"); return B2R_ERR_CUDA; }
+    if (!o || (n && (!d_bytes && total_bytes)) || (n && !d_offsets)) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
+    if (!aligned16(d_bytes)) { set_error("bytes must be 16-byte aligned"); return B2R_ERR_ALIGNMENT; }
+    int rc = check_outputs(c, o, true);
+    if (rc) return rc;
+    DeviceGuard g(c->device);
+    if (!g.ok) { set_error("cudaSetDevice(%d) failed", c->device); return B2R_ERR_CUDA; }
+    const uint64_t M = c->max_chars;
+    c->last_launches = 0;
+    CUDA_TRY(cudaMemsetAsync(c->scratch, 0, c->scratch_bytes, st));
+    WalkParams& pe = c->last;                                             // the emit stage over the N strings (and b2r_batch_result)
+    fill_walk_params(c, pe, d_bytes, d_offsets, n, total_bytes, o, M);
+    pe.fuse = 0; pe.fill_in_walk = 0; pe.prefilled = 0; pe.stagger_ns = 0;   // emit_kernel zero-fills the sparse columns itself
+    c->have_last = true;
+    bool wide = false;
+    for (uint32_t d = 0; d < c->n_defs; d++) wide = wide || c->packed[d].state_width == 2;
+    if (c->timing) CUDA_TRY(cudaEventRecord(c->ev[0], st));
+    if (n) {
+        if ((rc = c->ws_fmask.reserve(std::max<size_t>((size_t)pe.fm_words * n * 4, 16)))) return rc;
+        pe.fmask = (uint32_t*)c->ws_fmask.p;
+        for (uint32_t d = 0; d < c->n_defs; d++) {
+            if (pe.def[d].states) continue;
+            if ((rc = c->ws_states[d].reserve((size_t)n * o->row_pitch * (wide ? 2 : 1)))) return rc;
+            pe.def[d].states = c->ws_states[d].p;
+        }
+        // passes of whole strings: at most chunked_max_maps bytes (default 1 GiB) of slot transition vectors at a time, or one
+        // string's worth when that is more
+        const uint32_t K = (uint32_t)((M + LONG_CHUNK - 1) / LONG_CHUNK);
+        uint64_t s1_sum = 0;
+        uint32_t max_s1 = 0;
+        for (uint32_t d = 0; d < c->n_defs; d++) { s1_sum += c->packed[d].num_states + 1; max_s1 = std::max(max_s1, c->packed[d].num_states + 1); }
+        const uint64_t per_str = (uint64_t)K * s1_sum * 2;
+        const uint64_t cap = c->opt.chunked_max_maps > 0 ? (uint64_t)c->opt.chunked_max_maps : (1ull << 30);
+        uint64_t per_pass = std::min<uint64_t>(n, std::max<uint64_t>(1, cap / per_str));
+        per_pass = std::min<uint64_t>(per_pass, std::max<uint64_t>(1, (1ull << 31) / K));   // slot indices stay within u32
+        const uint32_t max_slots = (uint32_t)(per_pass * K);
+        const size_t nodes = long_level_nodes(max_slots);
+        size_t need = 0;
+        auto slot = [&](size_t bytes) { size_t off = need; need += align_up(bytes, 256); return off; };
+        size_t off_maps[B2R_MAX_DEFS], off_entry[B2R_MAX_DEFS];
+        for (uint32_t d = 0; d < c->n_defs; d++) {
+            off_maps[d] = slot(nodes * (c->packed[d].num_states + 1) * 2);
+            off_entry[d] = slot(nodes * 2);
+        }
+        const size_t off_uniq = slot((size_t)max_slots * 4 * 2), off_nuniq = slot(max_slots), off_which = slot((size_t)max_slots * max_s1);
+        if ((rc = c->ws_long.reserve(need))) return rc;
+        unsigned char* ws = (unsigned char*)c->ws_long.p;
+        LongParams lp;
+        memset(&lp, 0, sizeof lp);
+        lp.bytes = d_bytes; lp.n_defs = c->n_defs; lp.fused = 0;
+        lp.chunk_k = K; lp.max_chars = (uint32_t)M; lp.total_bytes = total_bytes;
+        lp.uniq = (uint16_t*)(ws + off_uniq); lp.n_uniq = ws + off_nuniq; lp.which = ws + off_which;
+        for (uint32_t d = 0; d < c->n_defs; d++) {
+            lp.def[d].byte_class = c->dev[d].byte_class; lp.def[d].trans = c->dev[d].trans;
+            lp.def[d].num_states = c->packed[d].num_states; lp.def[d].first_state = c->packed[d].first_state;
+            lp.def[d].num_classes = c->packed[d].num_classes;
+            lp.def[d].maps = (uint16_t*)(ws + off_maps[d]); lp.def[d].entry = (uint16_t*)(ws + off_entry[d]);
+        }
+        const size_t sb = wide ? 2 : 1;
+        for (uint64_t j0 = 0; j0 < n; j0 += per_pass) {
+            const uint64_t np = std::min<uint64_t>(per_pass, n - j0);
+            const uint32_t n_slots = (uint32_t)(np * K);
+            lp.n_chunks = n_slots; lp.str_offsets = d_offsets + j0;
+            if ((rc = launch_long_prepare(lp, st, &c->last_launches))) return rc;
+            WalkParams pw;
+            fill_walk_params(c, pw, d_bytes, d_offsets + j0, n_slots, total_bytes, o, LONG_CHUNK + 1);
+            pw.fuse = 0; pw.fill_in_walk = 0; pw.prefilled = 0; pw.stagger_ns = 0;
+            pw.chunk_k = K; pw.chunk_fm_words = pe.fm_words; pw.chunk_max_chars = (uint32_t)M; pw.chunk_stride = n;
+            pw.fmask = pe.fmask + j0;
+            for (uint32_t d = 0; d < c->n_defs; d++) {
+                pw.def[d].states = (unsigned char*)pe.def[d].states + j0 * o->row_pitch * sb;
+                pw.def[d].init_states = lp.def[d].entry;                  // level 0 of the tree
+            }
+            if ((rc = plan_walk(pw, wide, c->opt.force_table_mode, c->opt.force_hist_mode, c->opt.hist_cache_log2))) return rc;
+            if (j0)   // every walk hands out its tiles from a counter at 0
+                CUDA_TRY(cudaMemsetAsync((unsigned char*)c->scratch + offsetof(BatchCounters, tile_counter), 0, sizeof(unsigned long long), st));
+            if ((rc = launch_walk(pw, wide, st, nullptr))) return rc;
+            c->last_launches++;
+            pe.table_mode = pw.table_mode; pe.hist_mode = pw.hist_mode;   // b2r_last_plan reports the walk's placement
+        }
+    }
+    if (c->timing) CUDA_TRY(cudaEventRecord(c->ev[1], st));
+    if (n) {
+        if ((rc = launch_emit(pe, wide, st, nullptr))) return rc;
+        c->last_launches++;
+    }
+    if (c->timing) CUDA_TRY(cudaEventRecord(c->ev[2], st));
+    rc = enqueue_finalize(c, o, n, M, st);
+    if (rc) return rc;
+    if (c->timing) CUDA_TRY(cudaEventRecord(c->ev[3], st));
+    return B2R_OK;
+}
+
+int b2r_match_batch_chunked(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t total_bytes,
+                            const b2r_outputs* d_out, void* cuda_stream) {
+    if (!c) { set_error("null config"); return B2R_ERR_INVALID_ARG; }
+    return match_batch_chunked_impl(c, d_bytes, d_offsets, n, total_bytes, d_out, (cudaStream_t)cuda_stream);
+}
+
 uint32_t b2r_last_launch_count(const b2r_config* c) { return c ? c->last_launches : 0; }
 
 // testing / tuning hooks (the same knobs the B2R_* environment variables set when a handle is created)
@@ -610,6 +717,7 @@ int b2r_config_set_option(b2r_config* c, const char* name, const char* value) {
     else if (!strcmp(name, "sparse_direct")) o.sparse_direct = v;
     else if (!strcmp(name, "host_debug")) o.host_debug = v;
     else if (!strcmp(name, "long_fused")) o.long_fused = v;
+    else if (!strcmp(name, "chunked_max_maps")) o.chunked_max_maps = atoll(value);
     else { set_error("unknown option '%s'", name); return B2R_ERR_INVALID_ARG; }
     if (c->multi) return multi_set_option(c->multi, name, value);
     return B2R_OK;

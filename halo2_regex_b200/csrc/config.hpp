@@ -143,6 +143,7 @@ struct b2r_config {
         int host_threads = 0;         // sparse D2H mode: host worker threads (0 = default)
         int small_path = 1;           // 0: small batches take the sliced pipeline too (testing hook)
         int long_fused = 1;           // 0: the long-string path computes the chunk maps with the general multi-kernel pass (testing hook)
+        long long chunked_max_maps = 0;   // chunked batch: bytes of slot transition vectors per pass (0 = 1 GiB; testing hook)
         int sparse_cap = 0;           // sparse D2H mode: sectors per column slice before the dense fallback (0 = default; testing hook)
         int host_debug = 0;           // timing experiments only: 1 = skip the host-side clearing, 2 = skip the host-side scatter (results are wrong)
         int sparse_direct = 0;        // sparse D2H mode: 1 = the kernel stores the compacted sectors straight into pinned host memory (36-byte

@@ -140,12 +140,16 @@ static int plan_walk_tables(WalkParams& p, bool wide, int force_table_mode, int 
     return B2R_ERR_UNSUPPORTED;
 }
 
-template <int D>
+template <int D, bool CH>
 int launch_walk_d(const WalkParams& p, bool wide, size_t smem, int grid, int block, cudaStream_t st);
-template <> int launch_walk_d<1>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
-template <> int launch_walk_d<2>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
-template <> int launch_walk_d<3>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
-template <> int launch_walk_d<4>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
+template <> int launch_walk_d<1, false>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
+template <> int launch_walk_d<2, false>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
+template <> int launch_walk_d<3, false>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
+template <> int launch_walk_d<4, false>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
+template <> int launch_walk_d<1, true>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
+template <> int launch_walk_d<2, true>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
+template <> int launch_walk_d<3, true>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
+template <> int launch_walk_d<4, true>(const WalkParams&, bool, size_t, int, int, cudaStream_t);
 template <int D>
 int launch_emit_d(const WalkParams& p, bool wide, size_t smem, int grid, cudaStream_t st);
 template <> int launch_emit_d<1>(const WalkParams&, bool, size_t, int, cudaStream_t);
@@ -173,11 +177,12 @@ int launch_walk(const WalkParams& p, bool wide, void* stream, LaunchInfo* chosen
     const int grid = (int)(ctas < n_sm ? (ctas > 0 ? ctas : 1) : n_sm);
     if (chosen) { chosen->grid = grid; chosen->block = warps * 32; chosen->smem_bytes = smem; }
     cudaStream_t st = (cudaStream_t)stream;
+    const bool ch = p.chunk_k != 0;
     switch (p.n_defs) {
-        case 1: return launch_walk_d<1>(p, wide, smem, grid, warps * 32, st);
-        case 2: return launch_walk_d<2>(p, wide, smem, grid, warps * 32, st);
-        case 3: return launch_walk_d<3>(p, wide, smem, grid, warps * 32, st);
-        case 4: return launch_walk_d<4>(p, wide, smem, grid, warps * 32, st);
+        case 1: return ch ? launch_walk_d<1, true>(p, wide, smem, grid, warps * 32, st) : launch_walk_d<1, false>(p, wide, smem, grid, warps * 32, st);
+        case 2: return ch ? launch_walk_d<2, true>(p, wide, smem, grid, warps * 32, st) : launch_walk_d<2, false>(p, wide, smem, grid, warps * 32, st);
+        case 3: return ch ? launch_walk_d<3, true>(p, wide, smem, grid, warps * 32, st) : launch_walk_d<3, false>(p, wide, smem, grid, warps * 32, st);
+        case 4: return ch ? launch_walk_d<4, true>(p, wide, smem, grid, warps * 32, st) : launch_walk_d<4, false>(p, wide, smem, grid, warps * 32, st);
     }
     set_error("unsupported number of defs %u", p.n_defs);
     return B2R_ERR_UNSUPPORTED;

@@ -91,6 +91,14 @@ struct WalkParams {
     uint32_t spread_fill;            // 1: the fused zero-fill ops are issued across the chunk loop instead of in one burst per tile
     uint32_t stagger_ns;             // warp w of a CTA starts w * stagger_ns late: the warps' walk and emit phases interleave instead of coinciding
     uint32_t debug;                  // timing experiments only (B2R_DEBUG env): emit skips 1 zero-fill, 2 scan, 4 final-state loads, 8 status
+    // chunked batch mode (b2r_match_batch_chunked, walk_kernel<..., CH = true>): the "strings" are slots of LONG_CHUNK rows, slot k =
+    // chunk k % chunk_k of batch string k / chunk_k (offsets = the batch's string offsets).  A slot starts in init_states[k], stores its
+    // rows of the batch row (final state at the string's length, dummy after) and its two flag words in the batch layout
+    // (word w of slot c of string j at fmask[(2c + w) * chunk_stride + j])
+    uint32_t chunk_k;                // slots per string: ceil(M / LONG_CHUNK)
+    uint32_t chunk_fm_words;         // fm_words of the batch (M rows)
+    uint32_t chunk_max_chars;        // M of the batch (too-long rule, rows stored)
+    uint64_t chunk_stride;           // N of the whole batch (the flag-word stride)
 };
 
 constexpr uint32_t TABLE_REPL = 0;   // shared memory, one copy of every entry per bank (stride 128 B): conflict-free lookups

@@ -38,8 +38,17 @@ __device__ __forceinline__ uint32_t long_walk(const LongParams& p, uint32_t d, u
     return s;
 }
 __device__ __forceinline__ void long_chunk_range(const LongParams& p, uint32_t k, uint64_t& a, uint64_t& mid, uint64_t& b) {
-    a = (uint64_t)k * LONG_CHUNK;
-    b = a + LONG_CHUNK < p.len ? a + LONG_CHUNK : p.len;
+    if (p.chunk_k) {   // chunked batch: slot c of string j (a too-long string has no bytes, as in the batch walk)
+        const uint32_t j = k / p.chunk_k, c = k - j * p.chunk_k;
+        const uint64_t so = p.str_offsets[j], se = p.str_offsets[j + 1];
+        const uint64_t len = (se < so || se - so > (uint64_t)(p.max_chars - 1) || se > p.total_bytes) ? 0 : se - so;
+        const uint64_t s0 = (uint64_t)c * LONG_CHUNK;
+        a = so + (s0 < len ? s0 : len);
+        b = so + (s0 + LONG_CHUNK < len ? s0 + LONG_CHUNK : len);
+    } else {
+        a = (uint64_t)k * LONG_CHUNK;
+        b = a + LONG_CHUNK < p.len ? a + LONG_CHUNK : p.len;
+    }
     mid = a + LONG_HEAD < b ? a + LONG_HEAD : b;
 }
 
@@ -186,6 +195,16 @@ __global__ void __launch_bounds__(256) long_maps_gather_kernel(const __grid_cons
         long_chunk_range(p, k, a, mid, b);
         p.def[d].maps[t] = (uint16_t)(SMEM ? long_walk_s(p.bytes, mid, b, p.def[d].maps[t], cls_s, tr_s) : long_walk(p, d, p.def[d].maps[t], mid, b));
     }
+}
+
+// chunked batch: the map of every string's LAST slot becomes the constant map s -> first_state.  The composition over all slots
+// then starts every string in first_state, and every other slot gets the composition of its own string's earlier slots only
+// (no segmented scan); thread per (string, state)
+__global__ void __launch_bounds__(256) long_reset_kernel(uint16_t* maps, uint32_t n_strings, uint32_t chunk_k, uint32_t S1, uint32_t first) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (uint64_t)n_strings * S1) return;
+    const uint64_t j = t / S1, s = t - j * S1;
+    maps[((j + 1) * chunk_k - 1) * S1 + s] = (uint16_t)first;
 }
 
 // level l+1 map i = composition of its (up to 64) children at level l; thread per (node, state)
@@ -680,7 +699,7 @@ size_t long_level_nodes(uint32_t n_chunks) {
 // chunk offsets, chunk maps, the composition tree and the entry states of every chunk (level 0 of `entry`)
 int launch_long_prepare(const LongParams& lp, void* stream, uint32_t* launches) {
     cudaStream_t st = (cudaStream_t)stream;
-    if (!lp.fused) {   // the fused pass writes the chunk offsets itself
+    if (!lp.fused && !lp.chunk_k) {   // the fused pass writes the chunk offsets itself; the chunked batch walk reads the string offsets
         long_offsets_kernel<<<(lp.n_chunks + 1 + 255) / 256, 256, 0, st>>>(lp.offsets, lp.n_chunks, lp.len);
         LAUNCH_CHECK("long_offsets_kernel"); (*launches)++;
     }
@@ -737,6 +756,11 @@ int launch_long_prepare(const LongParams& lp, void* stream, uint32_t* launches) 
         if (smem_ok) long_maps_gather_kernel<true><<<grid_for(threads), 256, smem, st>>>(lp, d, lp.uniq, lp.n_uniq, lp.which);
         else long_maps_gather_kernel<false><<<grid_for(threads), 256, 0, st>>>(lp, d, lp.uniq, lp.n_uniq, lp.which);
         LAUNCH_CHECK("long_maps_gather_kernel"); (*launches)++;
+        if (lp.chunk_k) {
+            const uint32_t n_str = lp.n_chunks / lp.chunk_k;
+            long_reset_kernel<<<(unsigned)(((uint64_t)n_str * S1 + 255) / 256), 256, 0, st>>>(lp.def[d].maps, n_str, lp.chunk_k, S1, lp.def[d].first_state);
+            LAUNCH_CHECK("long_reset_kernel"); (*launches)++;
+        }
         // up the tree
         std::vector<uint32_t> n_level{lp.n_chunks};
         std::vector<size_t> off_level{0};

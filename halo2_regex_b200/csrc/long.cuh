@@ -48,6 +48,12 @@ struct LongParams {
     uint8_t* super;
     uint32_t* super_cnt;
     uint32_t fused;                      // 1: the fused pass is used (decided by long_plan)
+    // chunked batch (b2r_match_batch_chunked): chunk k is slot k % chunk_k of string k / chunk_k, whose bytes are
+    // [str_offsets[j], str_offsets[j+1]) (a string longer than max_chars - 1, or outside [0, total_bytes), has none); 0: one string
+    uint32_t chunk_k;
+    uint32_t max_chars;
+    const uint64_t* str_offsets;
+    uint64_t total_bytes;
 };
 
 constexpr uint32_t LONG_GROUP = 256;       // chunks per CTA of the fused prefix pass (16 warps share one copy of the replicated tables)

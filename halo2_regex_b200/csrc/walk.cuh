@@ -34,6 +34,7 @@
 #include "defs.hpp"
 #include "emit.cuh"
 #include "kernels.cuh"
+#include "long.cuh"
 
 namespace b2r {
 
@@ -139,7 +140,8 @@ __host__ __device__ inline size_t walk_smem_bytes(const WalkParams& p, uint32_t 
 }
 
 // TM: TABLE_REPL, TABLE_REPL16, TABLE_PLAIN, TABLE_PLAIN16 or TABLE_GLOBAL.  HM: HIST_SMEM or HIST_GLOBAL.
-template <int D, typename ST, int TM, int HM>
+// CH: chunked batch mode (kernels.cuh, chunk_k): the "strings" are LONG_CHUNK-row slots of the batch strings.
+template <int D, typename ST, int TM, int HM, bool CH = false>
 __global__ void __launch_bounds__(WALK_MAX_THREADS, 1) walk_kernel(const __grid_constant__ WalkParams p) {
     constexpr int DCH = WALK_DCH, PITCH = WALK_PITCH;
     constexpr int SB = sizeof(ST);
@@ -266,7 +268,7 @@ __global__ void __launch_bounds__(WALK_MAX_THREADS, 1) walk_kernel(const __grid_
 
     const uint32_t M = p.max_chars;
     const uint32_t Mpad = (M + 15u) & ~15u;                             // rows written (row_pitch >= Mpad by contract)
-    const uint32_t n_chunks = (Mpad + DCH - 1) / DCH;
+    const uint32_t n_chunks = CH ? LONG_CHUNK / DCH : (Mpad + DCH - 1) / DCH;   // a slot never stores a row past LONG_CHUNK
     const uint64_t rp = p.row_pitch;
     const uint32_t cls_lane_s = base_s + lay.cls + claneoff;
     uint32_t tabl[D], rowb[D], hist_s[D];
@@ -341,7 +343,19 @@ __global__ void __launch_bounds__(WALK_MAX_THREADS, 1) walk_kernel(const __grid_
         const uint64_t idx = tile_base + lane;
         const bool valid = idx < p.n_strings;
         uint64_t off = 0, end = 0;
-        if (valid) { off = p.offsets[idx]; end = p.offsets[idx + 1]; }
+        uint64_t ch_j = 0;                                              // chunked mode: the slot's string and chunk
+        uint32_t ch_c = 0;
+        bool ch_beyond = false;                                         // the slot starts past the string's final-state row
+        if (valid && CH) {
+            ch_j = idx / p.chunk_k; ch_c = (uint32_t)(idx - ch_j * p.chunk_k);
+            const uint64_t so = p.offsets[ch_j], se = p.offsets[ch_j + 1];
+            // a too-long string is walked as empty, as the batch walk does
+            const uint64_t len = (se < so || se - so > (uint64_t)(p.chunk_max_chars - 1) || se > p.total_bytes) ? 0 : se - so;
+            const uint64_t a = (uint64_t)ch_c * LONG_CHUNK;
+            ch_beyond = a > len;
+            off = so + (a < len ? a : len);
+            end = so + (a + LONG_CHUNK < len ? a + LONG_CHUNK : len);
+        } else if (valid) { off = p.offsets[idx]; end = p.offsets[idx + 1]; }
         // SURVEY 8(a) row 6: emit reports it; walk nothing.  Offsets that leave the byte buffer are treated the same way
         // (nothing outside [0, total_bytes) is ever read)
         const bool too_long = valid && (end < off || end - off > (uint64_t)(M - 1) || end > p.total_bytes);
@@ -352,7 +366,8 @@ __global__ void __launch_bounds__(WALK_MAX_THREADS, 1) walk_kernel(const __grid_
         uint32_t cur[D];
 #pragma unroll
         for (int d = 0; d < D; d++) {
-            const uint32_t f = (p.def[d].init_states && valid) ? (uint32_t)p.def[d].init_states[idx] : p.def[d].first_state;
+            uint32_t f = (p.def[d].init_states && valid) ? (uint32_t)p.def[d].init_states[idx] : p.def[d].first_state;
+            if (CH && ch_beyond) f = p.def[d].num_states;                 // dummy rows only
             cur[d] = E16 ? enc16(f) : (f << 16) | (f * stride);
         }
 
@@ -369,6 +384,20 @@ __global__ void __launch_bounds__(WALK_MAX_THREADS, 1) walk_kernel(const __grid_
             const uint64_t a = (roff & ~uint64_t(15)) + (uint32_t)kv * 16;
             in_ptr[i] = p.bytes + a;
             in_left[i] = rend > a ? (uint32_t)(rend - a) : 0u;
+        }
+        // chunked mode: where the rows of the slots this lane stores go in the batch columns, and how many of them there are
+        uint64_t ch_base[VPS];
+        uint32_t ch_rows[VPS];
+        if (CH) {
+            const uint32_t Mpad_b = (p.chunk_max_chars + 15u) & ~15u;
+#pragma unroll
+            for (int i = 0; i < VPS; i++) {
+                const int row = sr0 + (32 / VPS) * i;
+                const uint64_t j = __shfl_sync(0xffffffffu, ch_j, row);
+                const uint32_t c = __shfl_sync(0xffffffffu, ch_c, row);
+                ch_base[i] = j * rp + (uint64_t)c * LONG_CHUNK;
+                ch_rows[i] = Mpad_b - c * LONG_CHUNK < LONG_CHUNK ? Mpad_b - c * LONG_CHUNK : LONG_CHUNK;
+            }
         }
         const uint64_t tail_a = (off & ~uint64_t(15)) + DCH;            // extra vector of this lane's own row (unaligned strings)
         const uint8_t* const my_tail = p.bytes + tail_a;
@@ -580,14 +609,14 @@ __global__ void __launch_bounds__(WALK_MAX_THREADS, 1) walk_kernel(const __grid_
                 for (int i = 0; i < VPS; i++) {
                     const int row = sr0 + (32 / VPS) * i;
                     const uint32_t elem = cbase + (uint32_t)skv * (16 / SB);   // first row-element of this vector
-                    bool mine = row < (int)rows_here && elem < Mpad;
-                    if (p.segment_mode) {   // a chunk of a long string owns rows [0, len) only; the last chunk also the final-state row
+                    bool mine = row < (int)rows_here && elem < (CH ? ch_rows[i] : Mpad);
+                    if (!CH && p.segment_mode) {   // a chunk of a long string owns rows [0, len) only; the last chunk also the final-state row
                         const uint32_t rl = __shfl_sync(0xffffffffu, L, row);
                         mine = mine && (elem < rl || (tile_base + row + 1 == p.n_strings && elem < ((rl + 16u) & ~15u)));
                     }
                     if (mine) {
                         const uint4 v = lds128(INPLACE ? in_s + (chunk & 1) * (32 * PITCH) + row * PITCH + skv * 16 : st_s + (d * 32 + row) * SPITCH + skv * 16);
-                        *reinterpret_cast<uint4*>(col + ((tile_base + row) * rp + elem) * SB) = v;
+                        *reinterpret_cast<uint4*>(col + ((CH ? ch_base[i] : (tile_base + row) * rp) + elem) * SB) = v;
                     }
                 }
             }
@@ -596,7 +625,9 @@ __global__ void __launch_bounds__(WALK_MAX_THREADS, 1) walk_kernel(const __grid_
             if ((gcount & 31u) == 0 || chunk + 1 == n_chunks) {
                 const uint32_t wi = (gcount - 1) >> 5;
                 if (wi == 0) fw0 = fm; else if (wi == 1) fw1 = fm;
-                if (valid && wi < p.fm_words && (!p.fuse || wi >= 2)) p.fmask[(size_t)wi * p.n_strings + idx] = fm;
+                if (CH) {
+                    if (valid && 2 * ch_c + wi < p.chunk_fm_words) p.fmask[(size_t)(2 * ch_c + wi) * p.chunk_stride + ch_j] = fm;
+                } else if (valid && wi < p.fm_words && (!p.fuse || wi >= 2)) p.fmask[(size_t)wi * p.n_strings + idx] = fm;
                 fm = 0;
             }
             __syncwarp();

@@ -265,6 +265,18 @@ class RegexVerifyConfig:
         _raise(rc)
         return out
 
+    def match_batch_chunked_device(self, d_bytes, d_offsets, out, flags=0, stream=None):
+        """b2r_match_batch_chunked: the same call and the same outputs as match_batch_device, with every string cut into 1 KiB
+        chunks that are walked in parallel (batches of few, long strings).  Asynchronous on `stream`."""
+        import torch
+        if stream is None:
+            stream = torch.cuda.current_stream(d_bytes.device)
+        n = d_offsets.numel() - 1
+        st = out.struct(flags)
+        rc = lib.b2r_match_batch_chunked(self._h, d_bytes.data_ptr(), d_offsets.data_ptr(), n, d_bytes.numel(), C.byref(st), stream.cuda_stream)
+        _raise(rc)
+        return out
+
     def match_long_device(self, d_bytes, out, stream=None):
         """b2r_match_long: ONE string (the whole of `d_bytes`, a device tensor) with max_chars_size = len + 1; `out` is a
         DeviceOutputs(cfg, 1, max_chars_size=len + 1).  Asynchronous on `stream`."""

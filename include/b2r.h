@@ -129,7 +129,9 @@ uint32_t b2r_config_num_devices(const b2r_config*);
  *                                  default (1 for one def with replicated tables, else 2)
  *   stagger_ns   start offset between the warps of a walk CTA (-1: default)
  *   slices, host_threads, small_path, sparse_cap, sparse_direct, trace_host   host entry points (b2r_match_batch_host)
- *   hist_cache_log2, spread_fill, long_fused, debug, host_debug               kernel tuning / timing experiments */
+ *   hist_cache_log2, spread_fill, long_fused, debug, host_debug               kernel tuning / timing experiments
+ *   chunked_max_maps   b2r_match_batch_chunked: bytes of chunk transition vectors per pass (0: the default 1 GiB); small
+ *                      values force many passes */
 int b2r_config_set_option(b2r_config*, const char* name, const char* value);
 
 /* Page-locked host memory for the buffers handed to the host-pointer entry points (a copy into pageable memory cannot overlap
@@ -250,6 +252,18 @@ typedef struct b2r_outputs {
 int b2r_match_batch(b2r_config* cfg, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n_strings,
                     uint64_t total_bytes, const b2r_outputs* d_out, void* cuda_stream);
 int b2r_batch_result(b2r_config* cfg, void* cuda_stream, b2r_batch_status* out);
+
+/* Same contract as b2r_match_batch (device pointers, M = the handle's max_chars_size, asynchronous on cuda_stream, per-string
+ * problems in out->status, summarised by b2r_batch_result) — every defined output byte, status, record and counter is identical
+ * to what b2r_match_batch writes for the same call.  Strings are cut into 1 KiB chunks that are walked in parallel: for batches
+ * of few, long strings (b2r_match_batch gives each string one GPU lane; a few thousand strings do not fill the GPU).
+ * Workspace: the chunks' S-state transition vectors take ceil(M/1024) * (S+1) * 2 bytes per string and def; the strings are
+ * processed in passes of at most 1 GiB of them (at least one string per pass), so the handle keeps about that much device
+ * memory after a call with long strings and large DFAs.  No host copy or synchronisation inside the call: once a first call
+ * of the same shape has sized the workspace, the call can be captured in a CUDA graph.  b2r_last_launch_count, b2r_last_plan
+ * and the timing queries report on it (ms3[0] covers the transition vectors and the walk). */
+int b2r_match_batch_chunked(b2r_config* cfg, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n_strings,
+                            uint64_t total_bytes, const b2r_outputs* d_out, void* cuda_stream);
 
 /* Host-buffer variant (what a drop-in shim calls): copies bytes/offsets to the device, runs the kernels, copies
  * every requested column back, synchronises, and returns B2R_ERR_INVALID_TRANSITION / B2R_ERR_TOO_LONG when a
