@@ -578,6 +578,7 @@ int b2r_match_long(b2r_config* c, const uint8_t* d_bytes, uint64_t len, const b2
     WalkParams& pe = c->last;
     fill_walk_params(c, pe, d_bytes, d_offsets + n_chunks + 1, 1, len, o, M);
     pe.fuse = 0; pe.fill_in_walk = 0; pe.prefilled = 1;
+    pe.table_mode = pw.table_mode; pe.hist_mode = pw.hist_mode;           // b2r_last_plan reports the walk's placement
     pe.fmask = pw.fmask;
     for (uint32_t d = 0; d < c->n_defs; d++) pe.def[d].states = pw.def[d].states;
     c->have_last = true;

@@ -277,24 +277,26 @@ class RegexVerifyConfig:
         _raise(rc)
         return out
 
-    def match_long_device(self, d_bytes, out, stream=None):
+    def match_long_device(self, d_bytes, out, flags=0, stream=None):
         """b2r_match_long: ONE string (the whole of `d_bytes`, a device tensor) with max_chars_size = len + 1; `out` is a
-        DeviceOutputs(cfg, 1, max_chars_size=len + 1).  Asynchronous on `stream`."""
+        DeviceOutputs(cfg, 1, max_chars_size=len + 1); `flags`: B2R_OUT_* (B2R_OUT_ACCUMULATE_MULT adds into out's counters).
+        Asynchronous on `stream`."""
         import torch
         if stream is None:
             stream = torch.cuda.current_stream(d_bytes.device)
-        st = out.struct(0)
+        st = out.struct(flags)
         rc = lib.b2r_match_long(self._h, d_bytes.data_ptr(), d_bytes.numel(), C.byref(st), stream.cuda_stream)
         _raise(rc)
         return out
 
-    def match_long_host(self, data, out=None, check=True, **kw):
+    def match_long_host(self, data, out=None, flags=0, check=True, **kw):
         """b2r_match_long_host: ONE string (host bytes) through the chunked long-string path, max_chars_size = len + 1;
-        host buffers out (`out`: HostOutputs(1, len + 1, ...), allocated here if not given)."""
+        host buffers out (`out`: HostOutputs(1, len + 1, ...), allocated here if not given); `flags`: B2R_OUT_*
+        (B2R_OUT_ACCUMULATE_MULT adds into out's counters)."""
         data = np.ascontiguousarray(np.frombuffer(data, dtype=np.uint8) if isinstance(data, (bytes, bytearray)) else data, dtype=np.uint8)
         if out is None:
             out = HostOutputs(1, len(data) + 1, self.state_widths, self.table_num_rows, self.endpoint_num_rows, **kw)
-        st = out.struct(0)
+        st = out.struct(flags)
         res = _abi.BatchStatus()
         rc = lib.b2r_match_long_host(self._h, data.ctypes.data, len(data), C.byref(st), C.byref(res))
         if check:

@@ -122,7 +122,8 @@ int b2r_config_new_multi(const b2r_allstr* const* allstr, const b2r_substr* cons
                          uint32_t n_devices, b2r_config** out);
 uint32_t b2r_config_num_devices(const b2r_config*);
 /* testing / tuning knobs of a handle, the same ones the B2R_* environment variables set when it is created (none is needed in
- * production; results are bit-identical under every setting):
+ * production; results are bit-identical under every setting, except non-zero `debug` and `host_debug`, which skip work to time
+ * the rest and so produce wrong results):
  *   table_mode   repl | repl16 | plain | plain16 | global   placement of the walk tables (default: chosen by shared-memory budget)
  *   hist_mode    smem | global                              placement of the multiplicity bins
  *   fuse         1 | 2 | 0 | -1    emit stage inside walk_kernel / own kernel after a walk that zero-fills / own kernel that zero-fills too /
@@ -318,7 +319,8 @@ int b2r_last_kernel_ms(b2r_config*, float* walk_ms, float* total_ms);
 /* device time (ms) of the three stages of the last call: ms3[0] walk_kernel, ms3[1] emit_kernel, ms3[2] finalize_kernel */
 int b2r_last_stage_ms(b2r_config*, float* ms3);
 /* where the last call kept the walk tables (0 replicated shared memory, 1 shared memory, 2 global) and the
- * multiplicity bins (1 shared memory, 2 global) */
+ * multiplicity bins (1 shared memory, 2 global).  After b2r_match_long / b2r_match_long_host and b2r_match_batch_chunked:
+ * the placement of their walk over the chunks. */
 int b2r_last_plan(const b2r_config*, uint32_t* table_mode, uint32_t* hist_mode);
 
 #ifdef __cplusplus

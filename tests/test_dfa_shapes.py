@@ -219,17 +219,24 @@ def _padded(S):
 
 
 def _placement_expected(S, C, tm, hm, max_smem):
-    """One def, placement (tm, hm) forced: False = the planner cannot honour it (csrc/kernels.cu fits_k: the table entry holds
-    next * stride in 16 bits, REPL16 only up to 512 padded states, tables and shared-memory bins must fit, shared bins only with
-    u8 state columns); True = it fits with room to spare and must be honoured; None = too close to call from here."""
-    P, st = _padded(S), STRIDE[tm]
-    tables = C * P * st
-    table_ok = tm == "global" or (P * st <= 65536 and (tm != "repl16" or P <= 512) and tables <= max_smem)
-    bins = (S + 1) * 256 * 4
-    hist_ok = hm == "global" or (S <= 255 and bins <= max_smem)
+    """Placement (tm, hm) forced on defs with S states and C byte classes (ints for one def, lists for several): a tuple
+    (table_ok, hist_ok) with a False = the planner cannot honour that half (csrc/kernels.cu fits_k: every def's table entry holds
+    next * stride in 16 bits, REPL16 only up to 512 padded states, the tables of all defs and their shared-memory bins must fit,
+    shared bins only when no def needs a u16 state column, which then every def uses); True = it fits with room to spare and must
+    be honoured; None = too close to call from here."""
+    Ss, Cs = ([S], [C]) if isinstance(S, int) else (list(S), list(C))
+    Ps, st = [_padded(s) for s in Ss], STRIDE[tm]
+    tables = sum(c * P * st for c, P in zip(Cs, Ps))
+    table_ok = tm == "global" or (all(P * st <= 65536 and (tm != "repl16" or P <= 512) for P in Ps) and tables <= max_smem)
+    bins = sum((s + 1) * 256 * 4 for s in Ss)
+    # two or three defs on 16-bit entries may keep compact bins (fewer columns than 256): only their width rule is certain
+    compact = tm in ("plain16", "repl16") and 2 <= len(Ss) <= 3
+    hist_ok = hm == "global" or (max(Ss) <= 255 and (bins <= max_smem or compact))
     if not table_ok or not hist_ok:
         return (table_ok, hist_ok)
-    used = (tables + P * st + 256 * 128 if tm != "global" else 0) + (bins if hm == "smem" else 2048) + 64 * 1024
+    if hm == "smem" and bins > max_smem:
+        return None
+    used = (tables + len(Ps) * max(Ps) * st + 256 * 128 if tm != "global" else 0) + (bins if hm == "smem" else 2048 * len(Ss)) + 64 * 1024
     return True if used <= max_smem else None
 
 

@@ -263,15 +263,17 @@ def test_offset_warp_starts(monkeypatch):
     _both("three", 201, strings)
 
 
+FOUR_DEFS = [("regex1_test_lookup.txt", ["substr1_test_lookup.txt"]), ("regex2_test_lookup.txt", ["substr2_test_lookup.txt"]),
+             ("regex3_test_lookup.txt", ["substr3_test_lookup.txt"]), ("regex3_test_lookup.txt", ["substr1_test_lookup.txt", "substr2_test_lookup.txt"])]
+
+
 @pytest.mark.parametrize("fuse", [1, 2, 0])
 def test_four_defs(monkeypatch, fuse):
     """B2R_MAX_DEFS defs in one config (the emit kernel's per-thread scratch is at its largest)."""
     monkeypatch.setenv("B2R_FUSE", str(fuse))
-    spec = [("regex1_test_lookup.txt", ["substr1_test_lookup.txt"]), ("regex2_test_lookup.txt", ["substr2_test_lookup.txt"]),
-            ("regex3_test_lookup.txt", ["substr3_test_lookup.txt"]), ("regex3_test_lookup.txt", ["substr1_test_lookup.txt", "substr2_test_lookup.txt"])]
     rng = random.Random(404 + fuse)
     strings = _random_strings(rng, 400, 260, SNIPPETS) + [b"", b"x"]
-    _both(spec, 261, strings)
+    _both(FOUR_DEFS, 261, strings)
 
 
 def test_default_emit_placement():
