@@ -257,9 +257,18 @@ struct LaneString {
     uint32_t next_row;          // last examined row + 1; NO_POS = none yet / gap closed
     uint32_t carry_s, carry_ie; // id sum of row next_row-1, is_end_sum[next_row] (0 after a gap)
     uint32_t bw_t, sw[D], ew[D]; // bitmap words being assembled: rows [32*bw_t, 32*bw_t+32)
+    // Whole-sector stores of the records and compact bytes (SECTORS) and of the bitmaps (HOLD), DESIGN 4.2: one def only.  The
+    // stand-alone emit kernel of three defs, bound by its instructions, took 0.63 -> 0.98 ms with the extra stores, and the held
+    // bitmap words made the walk kernels of several defs spill.  The one-def stand-alone emit kernel keeps bitmap word stores
+    // (the same bytes; its walk counterpart is the fused kernel, where the sectors pay).  Whatever the choice, the fused and the
+    // stand-alone emit stage of a def set write the same bytes: the batch and chunked paths are compared tensor for tensor.
+    static constexpr bool SECTORS = D == 1;
+    static constexpr bool HOLD = SECTORS && !SG;
+    uint32_t hn, hk, hv[D][4];  // bitmap words held for the sectors of the span bw_t >> 3 (fold_bitmap_words)
+    uint32_t cbv[2];            // compact_pitch <= 8: the compact bytes, collected by write_masks, stored by store_compact
 
     __device__ __forceinline__ LaneString(const WalkParams& p_, const EmitTables<D>& tb_, uint64_t j_, const uint8_t* src_, uint32_t L_)
-        : p(p_), tb(tb_), j(j_), src(src_), L(L_), stash_g(NO_POS), stash_s(0) {}
+        : p(p_), tb(tb_), j(j_), src(src_), L(L_), stash_g(NO_POS), stash_s(0) { cbv[0] = 0; cbv[1] = 0; }
 
     __device__ __forceinline__ uint32_t entry(int d, uint32_t c, uint32_t s) const {
         const uint32_t S = p.def[d].num_states;
@@ -298,14 +307,66 @@ struct LaneString {
         }
         next_row = NO_POS; carry_s = 0; carry_ie = 0;
     }
-    __device__ __forceinline__ void flush_bitmap_words() {
-        if (bw_t == NO_POS) return;
+    // Bitmap words leave as whole sectors: the fill zeroed every sector long ago, so a word stored on its own would be a partial
+    // write of a sector that may have left L2.  The words of the 256-row span bw_t >> 3 that have a bit in some column are held
+    // (at most two: hk = their indices k0 | k1 << 3, hv = their values) and go out as one 32-byte sector per column when the scan
+    // leaves the span.  A third such word stores the sector at once and itself, and any later word of the span, word by word.
+    // Rows that are not 32-byte aligned take word stores throughout.
+    __device__ __forceinline__ bool bitmap_sectors(const uint8_t* col) const {
+        return (p.bitmap_pitch & 31) == 0 && (reinterpret_cast<uintptr_t>(col) & 31) == 0;
+    }
+    __device__ __forceinline__ void store_bitmap_sector(uint8_t* col, uint32_t v0, uint32_t v1) {
+        if (!col || (v0 | v1) == 0) return;
+        uint8_t* const sec = col + j * p.bitmap_pitch + 32ull * (bw_t >> 3);
+        const uint32_t k0 = hk & 7u, k1 = hn > 1 ? hk >> 3 : 8u;   // v1 == 0 unless two words are held
+        if (bitmap_sectors(col)) {
+            uint32_t w[8];
+#pragma unroll
+            for (int k = 0; k < 8; k++) w[k] = ((uint32_t)k == k0 ? v0 : 0u) | ((uint32_t)k == k1 ? v1 : 0u);
+            reinterpret_cast<uint4*>(sec)[0] = make_uint4(w[0], w[1], w[2], w[3]);
+            reinterpret_cast<uint4*>(sec)[1] = make_uint4(w[4], w[5], w[6], w[7]);
+        } else {
+            if (v0) reinterpret_cast<uint32_t*>(sec)[k0] = v0;
+            if (v1) reinterpret_cast<uint32_t*>(sec)[k1] = v1;
+        }
+    }
+    __device__ __forceinline__ void store_bitmap_held() {
 #pragma unroll
         for (int d = 0; d < D; d++) {
-            if (sw[d] && p.def[d].start_enable) *reinterpret_cast<uint32_t*>(p.def[d].start_enable + j * p.bitmap_pitch + 4 * bw_t) = sw[d];
-            if (ew[d] && p.def[d].end_enable) *reinterpret_cast<uint32_t*>(p.def[d].end_enable + j * p.bitmap_pitch + 4 * bw_t) = ew[d];
-            sw[d] = 0; ew[d] = 0;
+            store_bitmap_sector(p.def[d].start_enable, hv[d][0], hn > 1 ? hv[d][1] : 0u);
+            store_bitmap_sector(p.def[d].end_enable, hv[d][2], hn > 1 ? hv[d][3] : 0u);
         }
+    }
+    // the word being assembled is complete
+    __device__ __forceinline__ void fold_bitmap_words() {
+        uint32_t any = 0;
+#pragma unroll
+        for (int d = 0; d < D; d++) any |= sw[d] | ew[d];
+        if (any) {
+            if (HOLD && hn < 2) {
+#pragma unroll
+                for (int d = 0; d < D; d++) {
+                    if (hn == 0) { hv[d][0] = sw[d]; hv[d][2] = ew[d]; } else { hv[d][1] = sw[d]; hv[d][3] = ew[d]; }
+                }
+                hk |= (bw_t & 7u) << (3 * hn);
+                hn++;
+            } else {
+                if (HOLD && hn == 2) { store_bitmap_held(); hn = 3; }
+#pragma unroll
+                for (int d = 0; d < D; d++) {
+                    if (sw[d] && p.def[d].start_enable) *reinterpret_cast<uint32_t*>(p.def[d].start_enable + j * p.bitmap_pitch + 4 * bw_t) = sw[d];
+                    if (ew[d] && p.def[d].end_enable) *reinterpret_cast<uint32_t*>(p.def[d].end_enable + j * p.bitmap_pitch + 4 * bw_t) = ew[d];
+                }
+            }
+        }
+#pragma unroll
+        for (int d = 0; d < D; d++) { sw[d] = 0; ew[d] = 0; }
+    }
+    __device__ __forceinline__ void flush_bitmap_span() {
+        if (bw_t == NO_POS) return;
+        fold_bitmap_words();
+        if (HOLD && (hn == 1 || hn == 2)) store_bitmap_held();
+        hn = 0; hk = 0;
     }
     // flagged granule g; partner_flagged: the other granule of its 32-row window is flagged too (and writes itself)
     template <bool PATCH>
@@ -326,7 +387,10 @@ struct LaneString {
         uint32_t sidv[D][4];
 #pragma unroll
         for (int d = 0; d < D; d++) sidv[d][0] = sidv[d][1] = sidv[d][2] = sidv[d][3] = 0;
-        if (!PATCH && (g >> 1) != bw_t) { flush_bitmap_words(); bw_t = g >> 1; }
+        if (!PATCH && (g >> 1) != bw_t) {
+            if (bw_t != NO_POS && (g >> 4) == (bw_t >> 3)) fold_bitmap_words(); else flush_bitmap_span();
+            bw_t = g >> 1;
+        }
         while (hot) {
             const uint32_t r = (uint32_t)__ffs((int)hot) - 1u;
             hot &= hot - 1;
@@ -391,10 +455,14 @@ struct LaneString {
         bw_t = NO_POS;
 #pragma unroll
         for (int d = 0; d < D; d++) { sw[d] = 0; ew[d] = 0; }
+        hn = 0; hk = 0;
     }
     template <bool PATCH>
     __device__ __forceinline__ void scan_end() {
-        if (!invalid) { close_gap<PATCH>(); if (!PATCH) flush_bitmap_words(); }
+        if (!invalid) { close_gap<PATCH>(); if (!PATCH) flush_bitmap_span(); }
+        // an invalid string: the words finished before the failing row still go out, as word stores would have written them
+        // (the stand-alone emit kernel does), so that both emit paths leave the same bytes
+        else if (!PATCH && HOLD && (hn == 1 || hn == 2)) store_bitmap_held();
     }
     // fw0 / fw1: granule flags 0..63 of this string; further words come from the flag buffer `flags`
     template <bool PATCH>
@@ -468,7 +536,10 @@ struct LaneString {
 #pragma unroll
                     for (int w = 0; w < 8; w++)
                         if (q == (uint32_t)w) { mcv[w] |= c << sh; msv[w] |= sum << sh; }
-                    if (cb && n_cmp < p.compact_pitch) cb[n_cmp] = (uint8_t)c;
+                    if (cb && n_cmp < p.compact_pitch) {
+                        if (SECTORS && p.compact_pitch <= 8) { if (n_cmp < 4) cbv[0] |= c << (8 * n_cmp); else cbv[1] |= c << (8 * (n_cmp - 4)); }
+                        else cb[n_cmp] = (uint8_t)c;
+                    }
                     if (!in_run || sum != run_sum || i == a) {          // a new segment always starts a new run (the id sum changes at a boundary)
                         close_run(i);
                         in_run = true; run_start = i; run_sum = sum; run_coff = n_cmp;
@@ -479,6 +550,28 @@ struct LaneString {
             close_run(b);
         }
         flush();
+        // the last record ends in the first half of a sector: zeros in the second half, so that the sector leaves L2 whole
+        if (SECTORS && p.records && n_rec > 0 && n_rec < p.max_records) {
+            b2r_substr_record* const r = p.records + j * p.max_records + n_rec;
+            if ((reinterpret_cast<uintptr_t>(r) & 31) == 16) *reinterpret_cast<uint4*>(r) = make_uint4(0, 0, 0, 0);
+        }
+        // a compact area of more than 8 bytes that is not full: zeros up to its end (areas of at most 8: store_compact)
+        if (SECTORS && cb && p.compact_pitch > 8 && n_cmp > 0 && n_cmp < p.compact_pitch) {
+            for (uint32_t k = n_cmp; k < p.compact_pitch;) {
+                const uintptr_t a = reinterpret_cast<uintptr_t>(cb + k);
+                if ((a & 15) == 0 && k + 16 <= p.compact_pitch) { *reinterpret_cast<uint4*>(cb + k) = make_uint4(0, 0, 0, 0); k += 16; }
+                else if ((a & 3) == 0 && k + 4 <= p.compact_pitch) { *reinterpret_cast<uint32_t*>(cb + k) = 0u; k += 4; }
+                else { cb[k] = 0; k++; }
+            }
+        }
+    }
+    // compact_pitch <= 8: the string's whole compact area at once (the bytes write_masks collected, zeros after them).  Called by
+    // all lanes of a warp together, for neighbouring strings, so that the areas of four or more strings leave as whole sectors.
+    __device__ __forceinline__ void store_compact() {
+        uint8_t* const cb = p.compact_bytes + j * (uint64_t)p.compact_pitch;
+        if (p.compact_pitch == 8 && (reinterpret_cast<uintptr_t>(cb) & 7) == 0) *reinterpret_cast<uint2*>(cb) = make_uint2(cbv[0], cbv[1]);
+        else
+            for (uint32_t k = 0; k < p.compact_pitch; k++) cb[k] = (uint8_t)((k < 4 ? cbv[0] : cbv[1]) >> (8 * (k & 3)));
     }
 };
 
@@ -537,6 +630,10 @@ struct TileEmitter {
         if (__any_sync(FULL, patch)) {
             __syncwarp();
             if (patch) { ls.template scan<true>(fw0, fw1, p.fmask); r_nrec = ls.n_rec; r_ncmp = ls.n_cmp; }
+        }
+        if (LaneString<D, ST, SG>::SECTORS) {
+            __syncwarp();
+            if (p.compact_bytes && p.compact_pitch <= 8 && valid && !patch) ls.store_compact();
         }
         // two defs flagging one row: the string has no records (include/b2r.h), so no counts and no truncation flags either
         if (r_flags & B2R_ST_OVERLAP) { r_nrec = 0; r_ncmp = 0; }

@@ -645,7 +645,10 @@ __global__ void __launch_bounds__(128) long_emit_kernel(const __grid_constant__ 
         else {
             if (ls.overlap) r_flags = B2R_ST_OVERLAP;
             patch = ls.n_seg > EMIT_NSEG;
-            if (!patch) { ls.write_masks(); r_nrec = ls.n_rec; r_ncmp = ls.n_cmp; }
+            if (!patch) {
+                ls.write_masks(); r_nrec = ls.n_rec; r_ncmp = ls.n_cmp;
+                if (LaneString<D, ST>::SECTORS && p.compact_bytes && p.compact_pitch <= 8) ls.store_compact();
+            }
         }
     }
     if (__any_sync(0xffffffffu, patch)) {
