@@ -22,7 +22,7 @@ b2r_substr_transitions b2r_substr_start_states b2r_substr_end_states b2r_substr_
 b2r_config_new b2r_config_free b2r_config_num_defs b2r_config_max_chars_size b2r_config_device b2r_config_state_width
 b2r_config_dummy_state b2r_config_substr_id_offset b2r_config_num_byte_classes b2r_config_recommended_row_pitch
 b2r_config_recommended_bitmap_pitch b2r_table_num_rows b2r_table_rows b2r_endpoint_num_rows b2r_endpoint_rows
-b2r_match_batch b2r_match_batch_chunked b2r_batch_result b2r_match_batch_host b2r_match_substrs b2r_match_long b2r_match_long_host b2r_last_launch_count
+b2r_match_batch b2r_match_batch_chunked b2r_batch_result b2r_match_batch_host b2r_match_batch_chunked_host b2r_match_substrs b2r_match_long b2r_match_long_host b2r_last_launch_count
 b2r_config_set_timing b2r_last_kernel_ms b2r_last_stage_ms b2r_last_plan
 b2r_config_new_multi b2r_config_num_devices b2r_config_set_option b2r_host_alloc b2r_host_free b2r_host_register b2r_host_unregister
 b2r_last_host_bytes b2r_column_to_fr
@@ -79,6 +79,7 @@ def _load():
     sig("b2r_match_batch_chunked", i32, vp, vp, vp, u64, u64, C.POINTER(_abi.Outputs), vp)
     sig("b2r_batch_result", i32, vp, vp, C.POINTER(_abi.BatchStatus))
     sig("b2r_match_batch_host", i32, vp, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.BatchStatus))
+    sig("b2r_match_batch_chunked_host", i32, vp, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.BatchStatus))
     sig("b2r_match_substrs", i32, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.BatchStatus))
     sig("b2r_match_long", i32, vp, vp, u64, C.POINTER(_abi.Outputs), vp)
     sig("b2r_match_long_host", i32, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.BatchStatus))

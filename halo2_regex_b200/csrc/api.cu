@@ -590,13 +590,58 @@ int b2r_match_long(b2r_config* c, const uint8_t* d_bytes, uint64_t len, const b2
     return B2R_OK;
 }
 
+}  // extern "C"
+
+namespace b2r {
+
+// Workspace of one match_batch_chunked_impl call over n strings: the pass size, and where the slot transition vectors, the entry
+// states and the dedupe lists of a pass live in ws_long.  Every size grows with n.
+struct ChunkedLayout {
+    uint32_t K = 0, max_s1 = 0;
+    uint64_t per_pass = 0;
+    size_t off_maps[B2R_MAX_DEFS] = {}, off_entry[B2R_MAX_DEFS] = {}, off_uniq = 0, off_nuniq = 0, off_which = 0, need = 0;
+};
+static ChunkedLayout chunked_layout(const b2r_config* c, uint64_t n, uint64_t M) {
+    ChunkedLayout l;
+    // passes of whole strings: at most chunked_max_maps bytes (default 1 GiB) of slot transition vectors at a time, or one
+    // string's worth when that is more
+    l.K = (uint32_t)((M + LONG_CHUNK - 1) / LONG_CHUNK);
+    uint64_t s1_sum = 0;
+    for (uint32_t d = 0; d < c->n_defs; d++) { s1_sum += c->packed[d].num_states + 1; l.max_s1 = std::max(l.max_s1, c->packed[d].num_states + 1); }
+    const uint64_t per_str = (uint64_t)l.K * s1_sum * 2;
+    const uint64_t cap = c->opt.chunked_max_maps > 0 ? (uint64_t)c->opt.chunked_max_maps : (1ull << 30);
+    l.per_pass = std::min<uint64_t>(n, std::max<uint64_t>(1, cap / per_str));
+    l.per_pass = std::min<uint64_t>(l.per_pass, std::max<uint64_t>(1, (1ull << 31) / l.K));   // slot indices stay within u32
+    const uint32_t max_slots = (uint32_t)(l.per_pass * l.K);
+    const size_t nodes = long_level_nodes(max_slots);
+    auto slot = [&](size_t bytes) { size_t off = l.need; l.need += align_up(bytes, 256); return off; };
+    for (uint32_t d = 0; d < c->n_defs; d++) {
+        l.off_maps[d] = slot(nodes * (c->packed[d].num_states + 1) * 2);
+        l.off_entry[d] = slot(nodes * 2);
+    }
+    l.off_uniq = slot((size_t)max_slots * 4 * 2); l.off_nuniq = slot(max_slots); l.off_which = slot((size_t)max_slots * l.max_s1);
+    return l;
+}
+
+int chunked_reserve(b2r_config* c, uint64_t n, const b2r_outputs* o, uint64_t max_chars) {
+    if (!n) return B2R_OK;
+    bool wide = false;
+    for (uint32_t d = 0; d < c->n_defs; d++) wide = wide || c->packed[d].state_width == 2;
+    const uint64_t fm_words = (((max_chars - 1) + 15) / 16 + 31) / 32;   // as fill_walk_params
+    int rc;
+    if ((rc = c->ws_fmask.reserve(std::max<size_t>((size_t)fm_words * n * 4, 16)))) return rc;
+    for (uint32_t d = 0; d < c->n_defs; d++)
+        if (!o->states[d] && (rc = c->ws_states[d].reserve((size_t)n * o->row_pitch * (wide ? 2 : 1)))) return rc;
+    return c->ws_long.reserve(chunked_layout(c, n, max_chars).need);
+}
+
 // Chunked batch path: b2r_match_batch's outputs, with every string cut into K = ceil(M / LONG_CHUNK) slots that are walked in
 // parallel.  Per pass of whole strings: the slots' transition vectors (general prefix pass of long.cu), the last slot of every
 // string reset to the constant map -> first_state, the composition tree over all slots of the pass (entry state of every slot),
 // walk_kernel<..., CH = true> over the slots (state rows and flag words straight into the batch layout).  Then emit_kernel and
 // finalize_kernel over the N strings, exactly as match_batch_impl runs them when the emit stage is its own kernel.
-static int match_batch_chunked_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t total_bytes,
-                             const b2r_outputs* o, cudaStream_t st) {
+int match_batch_chunked_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t total_bytes,
+                             const b2r_outputs* o, uint64_t max_chars, cudaStream_t st) {
     if (c->device < 0) { set_error("this handle was created without a device (device = -1): no CPU fallback exists"); return B2R_ERR_CUDA; }
     if (!o || (n && (!d_bytes && total_bytes)) || (n && !d_offsets)) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
     if (!aligned16(d_bytes)) { set_error("bytes must be 16-byte aligned"); return B2R_ERR_ALIGNMENT; }
@@ -604,56 +649,36 @@ static int match_batch_chunked_impl(b2r_config* c, const uint8_t* d_bytes, const
     if (rc) return rc;
     DeviceGuard g(c->device);
     if (!g.ok) { set_error("cudaSetDevice(%d) failed", c->device); return B2R_ERR_CUDA; }
-    const uint64_t M = c->max_chars;
+    const uint64_t M = max_chars;
     c->last_launches = 0;
     CUDA_TRY(cudaMemsetAsync(c->scratch, 0, c->scratch_bytes, st));
     WalkParams& pe = c->last;                                             // the emit stage over the N strings (and b2r_batch_result)
     fill_walk_params(c, pe, d_bytes, d_offsets, n, total_bytes, o, M);
-    pe.fuse = 0; pe.fill_in_walk = 0; pe.prefilled = 0; pe.stagger_ns = 0;   // emit_kernel zero-fills the sparse columns itself
+    pe.fuse = 0; pe.fill_in_walk = 0; pe.stagger_ns = 0;
+    pe.prefilled = c->sparse_zeroed ? 1u : 0u;                            // else emit_kernel zero-fills the sparse columns itself
     c->have_last = true;
     bool wide = false;
     for (uint32_t d = 0; d < c->n_defs; d++) wide = wide || c->packed[d].state_width == 2;
     if (c->timing) CUDA_TRY(cudaEventRecord(c->ev[0], st));
     if (n) {
-        if ((rc = c->ws_fmask.reserve(std::max<size_t>((size_t)pe.fm_words * n * 4, 16)))) return rc;
+        if ((rc = chunked_reserve(c, n, o, M))) return rc;
         pe.fmask = (uint32_t*)c->ws_fmask.p;
-        for (uint32_t d = 0; d < c->n_defs; d++) {
-            if (pe.def[d].states) continue;
-            if ((rc = c->ws_states[d].reserve((size_t)n * o->row_pitch * (wide ? 2 : 1)))) return rc;
-            pe.def[d].states = c->ws_states[d].p;
-        }
-        // passes of whole strings: at most chunked_max_maps bytes (default 1 GiB) of slot transition vectors at a time, or one
-        // string's worth when that is more
-        const uint32_t K = (uint32_t)((M + LONG_CHUNK - 1) / LONG_CHUNK);
-        uint64_t s1_sum = 0;
-        uint32_t max_s1 = 0;
-        for (uint32_t d = 0; d < c->n_defs; d++) { s1_sum += c->packed[d].num_states + 1; max_s1 = std::max(max_s1, c->packed[d].num_states + 1); }
-        const uint64_t per_str = (uint64_t)K * s1_sum * 2;
-        const uint64_t cap = c->opt.chunked_max_maps > 0 ? (uint64_t)c->opt.chunked_max_maps : (1ull << 30);
-        uint64_t per_pass = std::min<uint64_t>(n, std::max<uint64_t>(1, cap / per_str));
-        per_pass = std::min<uint64_t>(per_pass, std::max<uint64_t>(1, (1ull << 31) / K));   // slot indices stay within u32
-        const uint32_t max_slots = (uint32_t)(per_pass * K);
-        const size_t nodes = long_level_nodes(max_slots);
-        size_t need = 0;
-        auto slot = [&](size_t bytes) { size_t off = need; need += align_up(bytes, 256); return off; };
-        size_t off_maps[B2R_MAX_DEFS], off_entry[B2R_MAX_DEFS];
-        for (uint32_t d = 0; d < c->n_defs; d++) {
-            off_maps[d] = slot(nodes * (c->packed[d].num_states + 1) * 2);
-            off_entry[d] = slot(nodes * 2);
-        }
-        const size_t off_uniq = slot((size_t)max_slots * 4 * 2), off_nuniq = slot(max_slots), off_which = slot((size_t)max_slots * max_s1);
-        if ((rc = c->ws_long.reserve(need))) return rc;
+        for (uint32_t d = 0; d < c->n_defs; d++)
+            if (!pe.def[d].states) pe.def[d].states = c->ws_states[d].p;
+        const ChunkedLayout l = chunked_layout(c, n, M);
+        const uint32_t K = l.K;
+        const uint64_t per_pass = l.per_pass;
         unsigned char* ws = (unsigned char*)c->ws_long.p;
         LongParams lp;
         memset(&lp, 0, sizeof lp);
         lp.bytes = d_bytes; lp.n_defs = c->n_defs; lp.fused = 0;
         lp.chunk_k = K; lp.max_chars = (uint32_t)M; lp.total_bytes = total_bytes;
-        lp.uniq = (uint16_t*)(ws + off_uniq); lp.n_uniq = ws + off_nuniq; lp.which = ws + off_which;
+        lp.uniq = (uint16_t*)(ws + l.off_uniq); lp.n_uniq = ws + l.off_nuniq; lp.which = ws + l.off_which;
         for (uint32_t d = 0; d < c->n_defs; d++) {
             lp.def[d].byte_class = c->dev[d].byte_class; lp.def[d].trans = c->dev[d].trans;
             lp.def[d].num_states = c->packed[d].num_states; lp.def[d].first_state = c->packed[d].first_state;
             lp.def[d].num_classes = c->packed[d].num_classes;
-            lp.def[d].maps = (uint16_t*)(ws + off_maps[d]); lp.def[d].entry = (uint16_t*)(ws + off_entry[d]);
+            lp.def[d].maps = (uint16_t*)(ws + l.off_maps[d]); lp.def[d].entry = (uint16_t*)(ws + l.off_entry[d]);
         }
         const size_t sb = wide ? 2 : 1;
         for (uint64_t j0 = 0; j0 < n; j0 += per_pass) {
@@ -690,10 +715,14 @@ static int match_batch_chunked_impl(b2r_config* c, const uint8_t* d_bytes, const
     return B2R_OK;
 }
 
+}  // namespace b2r
+
+extern "C" {
+
 int b2r_match_batch_chunked(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t total_bytes,
                             const b2r_outputs* d_out, void* cuda_stream) {
     if (!c) { set_error("null config"); return B2R_ERR_INVALID_ARG; }
-    return match_batch_chunked_impl(c, d_bytes, d_offsets, n, total_bytes, d_out, (cudaStream_t)cuda_stream);
+    return match_batch_chunked_impl(c, d_bytes, d_offsets, n, total_bytes, d_out, c->max_chars, (cudaStream_t)cuda_stream);
 }
 
 uint32_t b2r_last_launch_count(const b2r_config* c) { return c ? c->last_launches : 0; }

@@ -110,6 +110,8 @@ struct SparseMemo {
     std::vector<const void*> hosts;   // caller's buffer of every sparse column
     std::vector<uint32_t> cnt;        // [slice][column] sectors scattered
     std::vector<char> dense;          // [slice][column] 1: that column slice was copied densely
+    std::vector<uint64_t> cuts;       // slice i: strings [cuts[i], cuts[i + 1])
+    std::vector<size_t> idx_off;      // [slice][column] where its sector index list lies in the pinned arena
 };
 
 }  // namespace b2r
@@ -164,6 +166,7 @@ struct b2r_config {
     cudaStream_t in_stream = nullptr, out_stream = nullptr;   // host entry point: H2D / D2H copies overlapping the kernels
     cudaStream_t pay_stream = nullptr;                        // sparse D2H mode: the compacted sectors of a slice
     b2r::BatchCounters* counters_copy = nullptr;              // small-batch path: finalize_kernel leaves a copy of the batch counters here
+    bool sparse_zeroed = false;                               // chunked host pipeline: the sparse columns are zero already (emit_kernel skips its fill)
     static constexpr int MAX_SLICES = 16;
     cudaEvent_t ev_in[MAX_SLICES] = {}, ev_done[MAX_SLICES] = {}, ev_pay[MAX_SLICES] = {};
     b2r::BatchCounters* h_slices = nullptr;    // pinned: the counters of every slice of a host batch
@@ -183,6 +186,13 @@ void fill_walk_params(const b2r_config* c, WalkParams& p, const uint8_t* d_bytes
 int enqueue_finalize(b2r_config* c, const b2r_outputs* o, uint64_t n, uint64_t max_chars, cudaStream_t st);
 int match_batch_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t total_bytes, const b2r_outputs* o,
                      uint64_t max_chars, cudaStream_t st);
+// b2r_match_batch_chunked behind its argument checks; the same signature as match_batch_impl, so that the host pipeline can run either
+int match_batch_chunked_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t total_bytes, const b2r_outputs* o,
+                             uint64_t max_chars, cudaStream_t st);
+using BatchEntry = decltype(&match_batch_impl);
+// grows the workspaces a match_batch_chunked_impl call over n strings uses (ws_fmask, ws_states of the defs `o` has no state column
+// for, ws_long) to their size for n; a call over at most n strings then reserves nothing
+int chunked_reserve(b2r_config* c, uint64_t n, const b2r_outputs* o, uint64_t max_chars);
 void report_failure(const b2r_batch_status& r);      // sets the thread's error text for a failed string (reference panic text)
 // host.cu
 void multi_free(MultiState* m);

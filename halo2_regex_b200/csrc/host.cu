@@ -173,7 +173,7 @@ bool is_pinned(const void* h) {
 // Everything the call needs lives in ONE device arena (ws_cols) mirrored by ONE pinned host arena (pin_small):
 //   [offsets (n+1) u64 | input bytes | multiplicity block | BatchCounters copy | every requested column]
 // the first three parts go up in one copy, everything from the multiplicity block on comes back in one copy.
-int host_batch_small(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result) {
+int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result) {
     cudaStream_t st = c->host_stream;
     const bool trace = c->opt.trace_host;
     const auto wall0 = std::chrono::steady_clock::now();
@@ -236,7 +236,7 @@ int host_batch_small(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_of
     w_up = wall_us();
     dout.flags &= ~(uint32_t)B2R_OUT_SPARSE_D2H;                          // nothing to gain on one tile
     c->counters_copy = (BatchCounters*)(dv + off_cnt);
-    rc = match_batch_impl(c, dv + off_bytes, (const uint64_t*)(dv + off_offs), n, shift + nbytes, &dout, c->max_chars, st);
+    rc = entry(c, dv + off_bytes, (const uint64_t*)(dv + off_offs), n, shift + nbytes, &dout, c->max_chars, st);
     c->counters_copy = nullptr;
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(hv + off_mult, dv + off_mult, need - off_mult, cudaMemcpyDeviceToHost, st));
@@ -264,7 +264,15 @@ int host_batch_small(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_of
 }
 
 // ---- the sliced pipeline -------------------------------------------------------------------------------------------------------
-int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result,
+// What a host entry point runs on the device: `run` enqueues the kernels of one slice, and `by_bytes` selects the slicing that goes
+// with them (see `cuts` below) — the only other difference between b2r_match_batch_host and b2r_match_batch_chunked_host.
+struct DeviceEntry {
+    BatchEntry run;
+    bool by_bytes;                     // slices balanced by bytes at multiples of 4 strings (else by count, at multiples of 32)
+};
+const DeviceEntry BATCH_ENTRY = {match_batch_impl, false}, CHUNKED_ENTRY = {match_batch_chunked_impl, true};
+
+int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result,
                const MultiHook* hook) {
     if (!c || !ho || (n && !h_offsets)) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
     if (c->device < 0) { set_error("this handle was created without a device (device = -1): no CPU fallback exists"); return B2R_ERR_CUDA; }
@@ -286,7 +294,7 @@ int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets,
     const uint64_t nbytes = total - base;
     const uint64_t rp = ho->row_pitch, bp = ho->bitmap_pitch;
     if (!hook && c->opt.small_path && n >= 1 && n <= 32 && n * (rp * (4 + 3 * c->n_defs) + 2 * bp * c->n_defs) + nbytes <= (8u << 20))
-        return host_batch_small(c, h_bytes, h_offsets, n, ho, result);
+        return host_batch_small(c, entry.run, h_bytes, h_offsets, n, ho, result);
 
     if ((rc = c->ws_bytes.reserve(align_up(nbytes + 16, 256)))) return rc;
     if ((rc = c->ws_offsets.reserve((n + 1) * 8))) return rc;
@@ -364,11 +372,45 @@ int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets,
     unsigned char* const d_in = (unsigned char*)c->ws_bytes.p + (base & 15);
     const uint8_t* d_bytes = d_in - base;
     const uint64_t* d_offsets = (const uint64_t*)c->ws_offsets.p;
-    int n_slices = n >= 16384 ? (n >= (1u << 19) ? 16 : 8) : 1;
-    if (c->opt.slices >= 1 && c->opt.slices <= b2r_config::MAX_SLICES && n >= 16384) n_slices = c->opt.slices;   // testing hook
-    // slice boundaries are multiples of 32 strings: whole tiles per slice, and lo * pitch keeps the 16-byte alignment of every
-    // column for any legal pitch (bitmap_pitch is only a multiple of 4)
-    auto cut = [&](int k) { return k >= n_slices ? n : (n * (uint64_t)k / n_slices) & ~uint64_t(31); };   // (small first slices were tried: no gain)
+    const bool chunked = entry.by_bytes;
+    const bool forced = c->opt.slices >= 1 && c->opt.slices <= b2r_config::MAX_SLICES;   // testing hook
+    std::vector<uint64_t> cuts;                                           // slice i: strings [cuts[i], cuts[i + 1])
+    int n_slices;
+    if (!chunked) {
+        n_slices = n >= 16384 ? (n >= (1u << 19) ? 16 : 8) : 1;
+        if (forced && n >= 16384) n_slices = c->opt.slices;
+        // slice boundaries are multiples of 32 strings: whole tiles per slice, and lo * pitch keeps the 16-byte alignment of every
+        // column for any legal pitch (bitmap_pitch is only a multiple of 4)   (small first slices were tried: no gain)
+        for (int k = 0; k <= n_slices; k++) cuts.push_back(k >= n_slices ? n : (n * (uint64_t)k / n_slices) & ~uint64_t(31));
+    } else {
+        // Few long strings: slices balanced by BYTES, so that a batch of a few hundred strings overlaps H2D, kernels and D2H too.
+        // A slice holds at least 8 MiB of input (about 0.2 ms of H2D and several times that of D2H at PCIe 5 x16 rates, against
+        // some 20 launches of fixed cost per slice) and at least 32 strings (the emit stage gives a warp 32 strings), 16 at most.
+        n_slices = (int)std::max<uint64_t>(1, std::min<uint64_t>({(uint64_t)b2r_config::MAX_SLICES, nbytes >> 23, n / 32}));
+        if (forced) n_slices = c->opt.slices;
+        // Boundaries are multiples of 4 strings.  lo * bitmap_pitch is then a multiple of 16 (bitmap_pitch % 4 == 0), lo * row_pitch
+        // too (row_pitch % 16 == 0): every column slice keeps the 16-byte alignment check_outputs asks for and the emit stage's
+        // TMA zero-fill needs.  Nothing else depends on the slice base: every store of the emit stage (emit.cuh) stays inside the
+        // rows, records, status and compact area of its own string, and its whole-sector stores are chosen at run time from the
+        // actual address (bitmap words, status) or only pad a string's own area (records, compact bytes) — so no store reaches a
+        // neighbouring slice whose columns may be on their way to the host already.
+        cuts.push_back(0);
+        for (int k = 1; k < n_slices; k++) {
+            const uint64_t target = base + nbytes / n_slices * k + nbytes % n_slices * k / n_slices;
+            const uint64_t j = (uint64_t)(std::lower_bound(h_offsets, h_offsets + n + 1, target) - h_offsets);
+            cuts.push_back(std::max(cuts.back(), std::min(n, (j + 2) & ~uint64_t(3))));
+        }
+        cuts.push_back(n);
+        cuts.erase(std::unique(cuts.begin(), cuts.end()), cuts.end());    // no empty slices (a forced count larger than the batch)
+        if (cuts.size() < 2) cuts.push_back(n);
+        n_slices = (int)cuts.size() - 1;
+        // the workspaces of every slice, sized for the largest one before anything is enqueued (a buffer that grows between two
+        // slices would be freed under the kernels of the previous one)
+        uint64_t widest = 0;
+        for (int i = 0; i < n_slices; i++) widest = std::max(widest, cuts[i + 1] - cuts[i]);
+        if ((rc = chunked_reserve(c, widest, &dout, c->max_chars))) return rc;
+    }
+    auto cut = [&](int k) { return cuts[k]; };
 
     // ---- sparse mode: compaction arenas (device + pinned mirror) and the host threads ---------------------------------------------
     std::vector<const Copy*> scols;
@@ -389,7 +431,9 @@ int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets,
                 s.bytes = ni * scols[k]->stride;
                 s.n_sectors = (s.bytes + 31) / 32;
                 if (s.n_sectors > 0xFFFFFFFFull) { set_error("sparse D2H: a slice of more than 2^32 sectors"); return B2R_ERR_UNSUPPORTED; }
-                s.cap = (uint32_t)std::min<uint64_t>(s.n_sectors, 2 * ni + 1024);   // a sector or two per string and column; more -> dense copy
+                // a sector or two per string, column and KiB of row (rows of about 1 KiB on the batch path); more -> dense copy
+                const uint64_t per_string = chunked ? 2 * ((rp + 1023) / 1024) : 2;
+                s.cap = (uint32_t)std::min<uint64_t>(s.n_sectors, per_string * ni + 1024);
                 if (c->opt.sparse_cap > 0) s.cap = (uint32_t)std::min<uint64_t>(s.n_sectors, (uint64_t)c->opt.sparse_cap);
                 s.idx_off = sslot((size_t)s.cap * 4);
                 s.pay_off = sslot((size_t)s.cap * 32);
@@ -403,24 +447,24 @@ int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets,
         if (!c->opt.sparse_direct && (rc = c->ws_sparse_arena.reserve(sp_need + 256))) return rc;
         if (!c->pool) c->pool.reset(new HostPool(c->opt.host_threads > 0 ? (unsigned)c->opt.host_threads : default_host_threads()));
         CUDA_TRY(cudaMemsetAsync(c->ws_sparse.p, 0, n_sc * n_slices * sizeof(unsigned int), st));
-        // B2R_OUT_SPARSE_REUSE: these are the buffers the previous call filled (same batch geometry, hence the same arena layout):
-        // only the sectors it scattered are non-zero, and their index lists are still in the pinned arena
+        // B2R_OUT_SPARSE_REUSE: these are the buffers the previous call filled (same strings per buffer and pitches): only the sectors
+        // it scattered are non-zero, and their index lists are still in the pinned arena, where the memo says (its slices need not be
+        // this call's: the chunked pipeline cuts by bytes)
         SparseMemo& memo = c->sparse_memo;
-        reuse = (ho->flags & B2R_OUT_SPARSE_REUSE) && memo.valid && memo.n == n && memo.rp == rp && memo.bp == bp && memo.n_slices == n_slices &&
+        reuse = (ho->flags & B2R_OUT_SPARSE_REUSE) && memo.valid && memo.n == n && memo.rp == rp && memo.bp == bp &&
                 memo.sparse_cap == c->opt.sparse_cap && memo.hosts.size() == n_sc && c->pin_sparse[memo.arena].p;
         for (size_t k = 0; reuse && k < n_sc; k++) reuse = memo.hosts[k] == scols[k]->host;
         memo.valid = false;                                               // until this call has completed
         if (reuse && (c->opt.host_debug & 1)) {
         } else if (reuse) {
             const uint32_t piece = 1u << 16;
-            for (int i = 0; i < n_slices; i++)
+            for (int i = 0; i < memo.n_slices; i++)
                 for (size_t k = 0; k < n_sc; k++) {
-                    const SliceCol& s = sc[i * n_sc + k];
-                    unsigned char* dst = (unsigned char*)scols[k]->host + cut(i) * scols[k]->stride;
-                    const uint64_t bytes = s.bytes;
+                    unsigned char* dst = (unsigned char*)scols[k]->host + memo.cuts[i] * scols[k]->stride;
+                    const uint64_t bytes = (memo.cuts[i + 1] - memo.cuts[i]) * scols[k]->stride;
                     if (memo.dense[i * n_sc + k]) { c->pool->submit([dst, bytes] { memset(dst, 0, bytes); }); continue; }
                     const uint32_t cnt = memo.cnt[i * n_sc + k];
-                    const uint32_t* idx = (const uint32_t*)((unsigned char*)c->pin_sparse[memo.arena].p + s.idx_off);
+                    const uint32_t* idx = (const uint32_t*)((unsigned char*)c->pin_sparse[memo.arena].p + memo.idx_off[i * n_sc + k]);
                     for (uint32_t e0 = 0; e0 < cnt; e0 += piece)
                         c->pool->submit([=] {
                             const uint32_t e1 = std::min(cnt, e0 + piece);
@@ -462,6 +506,7 @@ int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets,
     uint64_t h2d = 0, d2h = 0;
     if (n) { CUDA_TRY(cudaMemcpyAsync(c->ws_offsets.p, h_offsets, (n + 1) * 8, cudaMemcpyHostToDevice, c->in_stream)); h2d += (n + 1) * 8; }
     std::vector<WalkParams> slice_params(n_slices);
+    uint32_t launches = 0;                                                // every kernel of the call, slices and sparse mode
     std::vector<uint64_t> slice_lo(n_slices);
     int n_sm = 148, max_smem = 0;
     device_limits(&n_sm, &max_smem);
@@ -486,11 +531,24 @@ int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets,
         if (ds.records) ds.records += lo * (size_t)ho->max_records;
         if (ds.compact_bytes) ds.compact_bytes += lo * (size_t)ho->compact_pitch;
         if (i > 0 || hook) ds.flags |= B2R_OUT_ACCUMULATE_MULT;          // the multiplicities of the slices add up
+        if (entry.by_bytes && ni) {
+            // the slice's sparse columns are zeroed by memsets over the whole GPU: emit_kernel would zero them from the warps that
+            // own their tiles, and a slice of a few hundred long strings has only a few tiles (2048 x 64 KiB in 16 slices, sparse
+            // D2H, B200: 16.5 ms per call with the emit stage's fill, 10.0 ms with the memsets)
+            auto zero = [&](void* p, size_t pitch) { return p ? cudaMemsetAsync(p, 0, ni * pitch, st) : cudaSuccess; };
+            for (uint32_t d = 0; d < c->n_defs; d++) {
+                CUDA_TRY(zero(ds.substr_ids[d], rp)); CUDA_TRY(zero(ds.start_enable[d], bp)); CUDA_TRY(zero(ds.end_enable[d], bp));
+            }
+            CUDA_TRY(zero(ds.masked_chars, rp)); CUDA_TRY(zero(ds.masked_substr_ids, rp));
+            c->sparse_zeroed = true;
+        }
         c->counters_copy = c->h_slices + i;                              // finalize_kernel leaves the slice's counters in pinned host memory
-        rc = match_batch_impl(c, d_bytes, d_offsets + lo, ni, total, &ds, c->max_chars, st);
+        rc = entry.run(c, d_bytes, d_offsets + lo, ni, total, &ds, c->max_chars, st);
         c->counters_copy = nullptr;
+        c->sparse_zeroed = false;
         if (rc) return rc;
         slice_params[i] = c->last;
+        launches += c->last_launches;
         if (sparse && ni)
             for (size_t k = 0; k < n_sc; k++) {
                 const SliceCol& s = sc[i * n_sc + k];
@@ -498,10 +556,12 @@ int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets,
                 sparsify_kernel<<<grid, 256, 0, st>>>((const uint4*)(cb + scols[k]->off + lo * scols[k]->stride), s.n_sectors, (uint32_t*)(sp_dev + s.idx_off),
                                                       (uint4*)(sp_dev + s.pay_off), s.cap, d_cnt + i * n_sc + k);
                 CUDA_TRY(cudaGetLastError());
+                launches++;
             }
         if (sparse && n_sc) {
             publish_counts_kernel<<<1, 32, 0, st>>>(d_cnt + i * n_sc, (unsigned int*)(sp_host + cnt_off) + i * n_sc, (uint32_t)n_sc);
             CUDA_TRY(cudaGetLastError());
+            launches++;
         }
         CUDA_TRY(cudaEventRecord(c->ev_done[i], st));
         if (trace && i == n_slices - 1) CUDA_TRY(cudaEventRecord(tev[1], c->in_stream));
@@ -608,6 +668,9 @@ int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets,
         for (size_t k = 0; k < n_sc; k++) memo.hosts.push_back(scols[k]->host);
         memo.cnt.assign(h_cnt, h_cnt + n_sc * n_slices);
         memo.dense = dense;
+        memo.cuts = cuts;
+        memo.idx_off.clear();
+        for (const SliceCol& s : sc) memo.idx_off.push_back(s.idx_off);
         memo.arena = arena;
         memo.valid = true;
     }
@@ -628,6 +691,7 @@ int host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets,
         for (auto& e : tev) cudaEventDestroy(e);
     }
     c->last_h2d_bytes = h2d; c->last_d2h_bytes = d2h + (uint64_t)n_slices * sizeof(BatchCounters);
+    if (chunked) c->last_launches = launches;                             // (b2r_match_batch_host keeps reporting its last slice)
 
     // the batch result: the lowest failing string over all slices (reference: the first panic), overlaps summed
     b2r_batch_status r;
@@ -682,20 +746,22 @@ int multi_set_option(MultiState* m, const char* name, const char* value) {
 
 namespace {
 
-int multi_host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result) {
+int multi_host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result) {
     MultiState* m = c->multi;
     const int nd = (int)m->kids.size();
     if (!ho || (n && !h_offsets)) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
     for (uint64_t j = 0; j < n; j++)
         if (h_offsets[j + 1] < h_offsets[j]) { set_error("offsets must be non-decreasing (string %llu)", (unsigned long long)j); return B2R_ERR_INVALID_ARG; }
-    // contiguous string ranges balanced by bytes, cut at multiples of 32 strings (whole tiles; column alignment)
+    // contiguous string ranges balanced by bytes, cut at multiples of 32 strings (whole tiles; column alignment) — of 4 strings for
+    // the chunked variant, whose slices have the same granularity (host_batch), so that a few long strings still reach every device
+    const uint64_t g = entry.by_bytes ? 4 : 32;
     std::vector<uint64_t> cutp(nd + 1, n);
     cutp[0] = 0;
     const uint64_t b0 = n ? h_offsets[0] : 0, total = n ? h_offsets[n] - b0 : 0;
     for (int k = 1; k < nd; k++) {
         const uint64_t target = b0 + total / nd * k + total % nd * k / nd;
         uint64_t j = (uint64_t)(std::lower_bound(h_offsets, h_offsets + n + 1, target) - h_offsets);
-        j = std::min(n, (j + 16) & ~uint64_t(31));
+        j = std::min(n, (j + g / 2) & ~(g - 1));
         cutp[k] = std::max(j, cutp[k - 1]);
     }
     const uint64_t rp = ho->row_pitch, bp = ho->bitmap_pitch;
@@ -724,7 +790,7 @@ int multi_host_batch(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_of
             hook.comm = m->comms[k]; hook.all_reduce = m->all_reduce; hook.error_string = m->error_string; hook.first = k == 0;
             memset(&res[k], 0, sizeof res[k]);
             static const uint64_t zero_off[1] = {0};
-            rcs[k] = host_batch(kid, h_bytes, n ? h_offsets + lo : zero_off, hi - lo, &o, &res[k], &hook);
+            rcs[k] = host_batch(kid, entry, h_bytes, n ? h_offsets + lo : zero_off, hi - lo, &o, &res[k], &hook);
             if (rcs[k]) errs[k] = get_error();
         });
     for (auto& t : threads) t.join();
@@ -790,15 +856,22 @@ uint32_t b2r_config_num_devices(const b2r_config* c) { return !c ? 0 : c->multi 
 int b2r_match_batch_host(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
                          b2r_batch_status* result) {
     if (!c) { set_error("null config"); return B2R_ERR_INVALID_ARG; }
-    if (c->multi) return multi_host_batch(c, h_bytes, h_offsets, n, ho, result);
-    return host_batch(c, h_bytes, h_offsets, n, ho, result, nullptr);
+    if (c->multi) return multi_host_batch(c, BATCH_ENTRY, h_bytes, h_offsets, n, ho, result);
+    return host_batch(c, BATCH_ENTRY, h_bytes, h_offsets, n, ho, result, nullptr);
+}
+
+int b2r_match_batch_chunked_host(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
+                                 b2r_batch_status* result) {
+    if (!c) { set_error("null config"); return B2R_ERR_INVALID_ARG; }
+    if (c->multi) return multi_host_batch(c, CHUNKED_ENTRY, h_bytes, h_offsets, n, ho, result);
+    return host_batch(c, CHUNKED_ENTRY, h_bytes, h_offsets, n, ho, result, nullptr);
 }
 
 int b2r_match_substrs(b2r_config* c, const uint8_t* characters, uint64_t len, const b2r_outputs* h_out, b2r_batch_status* result) {
     if (!c || !h_out) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
     const uint64_t offsets[2] = {0, len};
     b2r_config* one = c->multi ? c->multi->kids[0] : c;                   // one string: one device
-    return host_batch(one, characters, offsets, 1, h_out, result, nullptr);
+    return host_batch(one, BATCH_ENTRY, characters, offsets, 1, h_out, result, nullptr);
 }
 
 int b2r_last_host_bytes(const b2r_config* c, uint64_t* h2d_bytes, uint64_t* d2h_bytes) {

@@ -232,6 +232,14 @@ class RegexVerifyConfig:
         """Host buffers in, host buffers out (H2D, kernels, D2H inside): the call a drop-in shim makes.
         sparse=True: B2R_OUT_SPARSE_D2H — the zero-dominated columns cross PCIe compacted and are expanded by host threads.
         reuse=True: B2R_OUT_SPARSE_REUSE — `out` is what the previous call on this handle filled: only its sectors are cleared."""
+        return self._host_call(lib.b2r_match_batch_host, data, offsets, out, flags, check, sparse, reuse, kw)
+
+    def match_batch_chunked_host(self, data, offsets, out=None, flags=0, check=True, sparse=False, reuse=False, **kw):
+        """b2r_match_batch_chunked_host: the call and the outputs of match_batch_host, with the kernels of
+        match_batch_chunked_device (every string cut into 1 KiB chunks walked in parallel) — for batches of few, long strings."""
+        return self._host_call(lib.b2r_match_batch_chunked_host, data, offsets, out, flags, check, sparse, reuse, kw)
+
+    def _host_call(self, fn, data, offsets, out, flags, check, sparse, reuse, kw):
         if sparse:
             flags |= _abi.B2R_OUT_SPARSE_D2H
         if reuse:
@@ -243,7 +251,7 @@ class RegexVerifyConfig:
             out = self.new_host_outputs(n, **kw)
         st = out.struct(flags)
         res = _abi.BatchStatus()
-        rc = lib.b2r_match_batch_host(self._h, data.ctypes.data, offsets.ctypes.data, n, C.byref(st), C.byref(res))
+        rc = fn(self._h, data.ctypes.data, offsets.ctypes.data, n, C.byref(st), C.byref(res))
         if check:
             _raise(rc, res)
         return out, res

@@ -272,6 +272,17 @@ int b2r_match_batch_chunked(b2r_config* cfg, const uint8_t* d_bytes, const uint6
 int b2r_match_batch_host(b2r_config* cfg, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n_strings,
                          const b2r_outputs* h_out, b2r_batch_status* result);
 
+/* Host-buffer variant of b2r_match_batch_chunked, for batches of few, long strings from host memory.  The contract is that of
+ * b2r_match_batch_host — arguments, return codes, *result, flags (B2R_OUT_SPARSE_D2H, B2R_OUT_SPARSE_REUSE, B2R_OUT_ACCUMULATE_MULT),
+ * pinned or pageable buffers, NULL columns, multi-device handles — and every defined output byte, status, record and counter is
+ * identical to what b2r_match_batch_host writes for the same call; the kernels are those of b2r_match_batch_chunked.  The batch
+ * is cut into slices balanced by bytes at multiples of 4 strings (b2r_match_batch_host: by count, at multiples of 32), so that
+ * a few hundred long strings also overlap the H2D copies, the kernels and the D2H copies; a multi-device handle splits the
+ * strings at multiples of 4 as well.  b2r_last_launch_count counts the kernels of every slice, b2r_last_host_bytes and
+ * b2r_last_plan report on the call as after b2r_match_batch_host. */
+int b2r_match_batch_chunked_host(b2r_config* cfg, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n_strings,
+                                 const b2r_outputs* h_out, b2r_batch_status* result);
+
 /* Single-string convenience with the exact shape of match_substrs (src/lib.rs:311-315): one &[u8] in,
  * M-row columns out (host pointers, row_pitch ignored -> M). */
 int b2r_match_substrs(b2r_config* cfg, const uint8_t* characters, uint64_t len, const b2r_outputs* h_out,
@@ -308,7 +319,9 @@ int b2r_match_long_host(b2r_config* cfg, const uint8_t* h_bytes, uint64_t len, c
 int b2r_column_to_fr(b2r_config* cfg, const void* d_col, uint32_t kind, const uint64_t* d_offsets, uint64_t n_strings, uint64_t rows,
                      uint64_t pitch, uint64_t* d_fr, void* cuda_stream);
 
-/* kernel launches enqueued by the last b2r_match_* call on this handle (for benchmark accounting) */
+/* kernel launches enqueued by the last b2r_match_* call on this handle (for benchmark accounting).  A sliced
+ * b2r_match_batch_host call (and b2r_match_substrs) reports the kernels of its LAST slice only; b2r_match_batch_chunked_host
+ * reports those of every slice plus the sparse-D2H kernels; a multi-device handle sums over its devices. */
 uint32_t b2r_last_launch_count(const b2r_config*);
 /* bytes the last host-pointer call moved over PCIe in each direction */
 int b2r_last_host_bytes(const b2r_config*, uint64_t* h2d_bytes, uint64_t* d2h_bytes);

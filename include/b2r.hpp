@@ -187,7 +187,9 @@ public:
         std::vector<b2r_string_status> status;
         std::vector<std::vector<uint64_t>> mult, endpoint_mult;
     };
-    BatchWitness match_batch(const std::vector<std::vector<uint8_t>>& strings, bool sparse_d2h = false) const {
+    // chunked: b2r_match_batch_chunked_host, the same outputs with every string cut into 1 KiB chunks walked in parallel (batches of
+    // few, long strings, such as e-mail bodies)
+    BatchWitness match_batch(const std::vector<std::vector<uint8_t>>& strings, bool sparse_d2h = false, bool chunked = false) const {
         const size_t M = max_chars_size, D = regex_defs.size(), n = strings.size();
         BatchWitness w;
         w.n = n; w.row_pitch = (M + 31) & ~size_t(31); w.bitmap_pitch = ((M + 7) / 8 + 31) & ~size_t(31);
@@ -208,7 +210,7 @@ public:
         w.masked_chars.resize(n * w.row_pitch); w.masked_substr_ids.resize(n * w.row_pitch); w.status.resize(n);
         out.masked_chars = w.masked_chars.data(); out.masked_substr_ids = w.masked_substr_ids.data(); out.status = w.status.data();
         b2r_batch_status res{};
-        const int rc = b2r_match_batch_host(h_.get(), bytes.data(), offsets.data(), n, &out, &res);
+        const int rc = (chunked ? b2r_match_batch_chunked_host : b2r_match_batch_host)(h_.get(), bytes.data(), offsets.data(), n, &out, &res);
         if (rc == B2R_ERR_INVALID_TRANSITION) throw InvalidTransition(res);
         detail::check(rc);
         return w;

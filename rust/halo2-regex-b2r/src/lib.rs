@@ -157,6 +157,14 @@ impl Config {
         if rc == B2R_OK { Ok(res) } else { Err((rc, res)) }
     }
 
+    /// `match_batch` for batches of few, long strings (e-mail bodies): the same arguments, result and outputs, with every string
+    /// cut into 1 KiB chunks that are walked in parallel on the device (`b2r_match_batch_chunked_host`).
+    pub fn match_batch_chunked(&self, bytes: &[u8], offsets: &[u64], out: &b2r_outputs) -> Result<b2r_batch_status, (i32, b2r_batch_status)> {
+        let mut res = b2r_batch_status::default();
+        let rc = unsafe { b2r_match_batch_chunked_host(self.ptr, bytes.as_ptr(), offsets.as_ptr(), offsets.len() as u64 - 1, out, &mut res) };
+        if rc == B2R_OK { Ok(res) } else { Err((rc, res)) }
+    }
+
     /// `RegexTableConfig::load` row order (reference src/table.rs:101-122): rows of {char, cur_state, next_state, substr_id};
     /// multiplicity counter r of `b2r_outputs.mult[d]` belongs to row r.
     pub fn table_rows(&self, d: usize) -> Vec<[u64; 4]> {

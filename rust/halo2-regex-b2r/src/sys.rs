@@ -73,6 +73,8 @@ extern "C" {
     pub fn b2r_match_substrs(c: *mut b2r_config, characters: *const u8, len: u64, out: *const b2r_outputs, result: *mut b2r_batch_status) -> c_int;
     pub fn b2r_match_batch_host(c: *mut b2r_config, bytes: *const u8, offsets: *const u64, n: u64, out: *const b2r_outputs,
                                 result: *mut b2r_batch_status) -> c_int;
+    pub fn b2r_match_batch_chunked_host(c: *mut b2r_config, bytes: *const u8, offsets: *const u64, n: u64, out: *const b2r_outputs,
+                                        result: *mut b2r_batch_status) -> c_int;
     pub fn b2r_match_batch(c: *mut b2r_config, d_bytes: *const u8, d_offsets: *const u64, n: u64, total_bytes: u64,
                            d_out: *const b2r_outputs, cuda_stream: *mut c_void) -> c_int;
     pub fn b2r_match_batch_chunked(c: *mut b2r_config, d_bytes: *const u8, d_offsets: *const u64, n: u64, total_bytes: u64,
