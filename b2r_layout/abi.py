@@ -89,7 +89,23 @@ class Outputs(C.Structure):
     ]
 
 
+class RowCount(C.Structure):
+    _fields_ = [("row", C.c_uint32), ("count", C.c_uint32)]
+
+
+class StringMultStruct(C.Structure):
+    """b2r_string_mult_outputs"""
+    _fields_ = [
+        ("max_entries", C.c_uint32),
+        ("reserved", C.c_uint32),
+        ("entries", C.c_void_p * B2R_MAX_DEFS),
+        ("n_entries", C.c_void_p * B2R_MAX_DEFS),
+        ("endpoint_counts", C.c_void_p * B2R_MAX_DEFS),
+    ]
+
+
 assert C.sizeof(StringStatus) == 32
+assert C.sizeof(RowCount) == 8
 assert C.sizeof(SubstrRecord) == 16
 assert C.sizeof(BatchStatus) == 32
 

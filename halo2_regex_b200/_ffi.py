@@ -26,6 +26,7 @@ b2r_match_batch b2r_match_batch_chunked b2r_batch_result b2r_match_batch_host b2
 b2r_config_set_timing b2r_last_kernel_ms b2r_last_stage_ms b2r_last_plan
 b2r_config_new_multi b2r_config_num_devices b2r_config_set_option b2r_host_alloc b2r_host_free b2r_host_register b2r_host_unregister
 b2r_last_host_bytes b2r_column_to_fr
+b2r_string_mult b2r_match_batch_host_mult b2r_match_batch_chunked_host_mult
 """.split()
 
 
@@ -97,6 +98,10 @@ def _load():
     sig("b2r_host_unregister", i32, vp)
     sig("b2r_last_host_bytes", i32, vp, pu64, pu64)
     sig("b2r_column_to_fr", i32, vp, vp, u32, vp, u64, u64, u64, vp, vp)
+    sig("b2r_string_mult", i32, vp, vp, vp, u64, u64, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.StringMultStruct), vp)
+    sig("b2r_match_batch_host_mult", i32, vp, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.StringMultStruct), C.POINTER(_abi.BatchStatus))
+    sig("b2r_match_batch_chunked_host_mult", i32, vp, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.StringMultStruct),
+        C.POINTER(_abi.BatchStatus))
     return L
 
 

@@ -24,7 +24,8 @@ int upload_tables(b2r_config* c) {
     for (uint32_t d = 0; d < c->n_defs; d++) {
         const PackedDef& pd = c->packed[d];
         total += align_up(256, 256) + align_up(pd.trans.size() * 4, 256) + align_up(pd.row_bin.size() * 4, 256) +
-                 2 * align_up(pd.erows.size() * 4, 256) + align_up((size_t)pd.num_classes * padded_states(pd.num_states) * 4, 256);
+                 2 * align_up(pd.erows.size() * 4, 256) + align_up((size_t)pd.num_classes * padded_states(pd.num_states) * 4, 256) +
+                 2 * align_up(pd.rows.size() * 4, 256);
     }
     total += 512;                                                          // the two byte <-> bin column maps
     CUDA_TRY(cudaMalloc(&c->tables, total));
@@ -50,6 +51,16 @@ int upload_tables(b2r_config* c) {
         c->dev[d].row_bin = (uint32_t*)put(pd.row_bin.data(), pd.row_bin.size() * 4);
         c->dev[d].erow_start_bin = (uint32_t*)put(pd.erow_start_bin.data(), pd.erows.size() * 4);
         c->dev[d].erow_end_bin = (uint32_t*)put(pd.erow_end_bin.data(), pd.erows.size() * 4);
+        {   // the per-string post-pass maps the few distinct bins of a string to rows by binary search (a dense 256 * S map would
+            // take 67 MB at S = 65535)
+            std::vector<std::pair<uint32_t, uint32_t>> br;
+            for (size_t r = 1; r < pd.rows.size(); r++) br.push_back({pd.row_bin[r], (uint32_t)r});
+            std::sort(br.begin(), br.end());
+            std::vector<uint32_t> bins, rows;
+            for (const auto& x : br) { bins.push_back(x.first); rows.push_back(x.second); }
+            c->dev[d].sorted_bins = (uint32_t*)put(bins.data(), bins.size() * 4);
+            c->dev[d].sorted_rows = (uint32_t*)put(rows.data(), rows.size() * 4);
+        }
         scratch += align_up((size_t)256 * pd.num_states * 8, 256) + 2 * align_up((size_t)std::max<uint32_t>(pd.num_substrs, 1) * pd.num_states * 8, 256);
     }
     {   // compact bins: a column for every byte that some def has a transition for, one more for all the others
@@ -409,7 +420,7 @@ void b2r_config_free(b2r_config* c) {
     if (c->device >= 0) {
         DeviceGuard g(c->device);
         cudaFree(c->tables); cudaFree(c->scratch); cudaFree(c->d_batch_status);
-        c->ws_fmask.release(); c->ws_long.release();
+        c->ws_fmask.release(); c->ws_long.release(); c->ws_smult.release();
         for (auto& b : c->ws_states) b.release();
         c->ws_bytes.release(); c->ws_offsets.release(); c->ws_cols.release(); c->ws_sparse.release(); c->ws_sparse_arena.release();
         c->pin_sparse[0].release(); c->pin_sparse[1].release(); c->pin_small.release();

@@ -63,6 +63,7 @@ struct DevDef {
     uint32_t* trans = nullptr;
     uint32_t* hot = nullptr;     // walk table [C][P] (walk.cuh)
     uint32_t *row_bin = nullptr, *erow_start_bin = nullptr, *erow_end_bin = nullptr;
+    uint32_t *sorted_bins = nullptr, *sorted_rows = nullptr;   // rows >= 1 ordered by bin ch*S + cur (string_mult.cu: bin -> row by binary search)
     unsigned long long *hist = nullptr, *ep_start = nullptr, *ep_end = nullptr;  // inside cfg->scratch
 };
 
@@ -154,6 +155,7 @@ struct b2r_config {
     b2r::DevBuf ws_fmask;                  // granule flags (walk -> emit)
     b2r::DevBuf ws_long;                   // long-string path: chunk offsets, transition-vector tree, entry states, flag summary
     b2r::DevBuf ws_states[B2R_MAX_DEFS];   // state column of a def the caller did not ask for (emit reads it)
+    b2r::DevBuf ws_smult;                  // per-string counters of strings longer than one string_mult segment (string_mult.cu)
     b2r::WalkParams last = {};
     bool have_last = false;
     uint32_t last_launches = 0;
@@ -194,6 +196,13 @@ using BatchEntry = decltype(&match_batch_impl);
 // for, ws_long) to their size for n; a call over at most n strings then reserves nothing
 int chunked_reserve(b2r_config* c, uint64_t n, const b2r_outputs* o, uint64_t max_chars);
 void report_failure(const b2r_batch_status& r);      // sets the thread's error text for a failed string (reference panic text)
+// string_mult.cu: the argument checks of the per-string outputs (host: pointers into host memory, states / status may be NULL),
+// and the post-pass over n strings whose state columns and status the match kernels have written (device pointers; `states` =
+// the columns they used, scratch ones included).  Adds its kernels to *launches.
+int check_string_mult(const b2r_config* c, const b2r_string_mult_outputs* sm);
+bool string_mult_wanted(const b2r_config* c, const b2r_string_mult_outputs* sm, uint32_t d);
+int string_mult_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t max_chars, void* const* states,
+                     uint64_t row_pitch, const b2r_string_status* status, const b2r_string_mult_outputs* sm, cudaStream_t st, uint32_t* launches);
 // host.cu
 void multi_free(MultiState* m);
 int multi_set_option(MultiState* m, const char* name, const char* value);

@@ -173,7 +173,8 @@ bool is_pinned(const void* h) {
 // Everything the call needs lives in ONE device arena (ws_cols) mirrored by ONE pinned host arena (pin_small):
 //   [offsets (n+1) u64 | input bytes | multiplicity block | BatchCounters copy | every requested column]
 // the first three parts go up in one copy, everything from the multiplicity block on comes back in one copy.
-int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result) {
+int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
+                     const b2r_string_mult_outputs* sm, b2r_batch_status* result) {
     cudaStream_t st = c->host_stream;
     const bool trace = c->opt.trace_host;
     const auto wall0 = std::chrono::steady_clock::now();
@@ -206,6 +207,18 @@ int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, co
     const size_t o_st = want(ho->status, n * sizeof(b2r_string_status));
     const size_t o_rec = want(ho->records, n * (size_t)ho->max_records * sizeof(b2r_substr_record));
     const size_t o_cb = want(ho->compact_bytes, n * (size_t)ho->compact_pitch);
+    // per-string counts: they come back with the columns; the entry slots go up first (the post-pass leaves unused slots alone)
+    bool want_sm = false;
+    b2r_string_mult_outputs dsm{};
+    size_t o_ent[B2R_MAX_DEFS] = {}, o_nent[B2R_MAX_DEFS] = {}, o_epc[B2R_MAX_DEFS] = {};
+    for (uint32_t d = 0; d < c->n_defs; d++) {
+        if (!string_mult_wanted(c, sm, d)) continue;
+        want_sm = true;
+        o_ent[d] = want(sm->entries[d], n * (size_t)sm->max_entries * sizeof(b2r_row_count));
+        o_nent[d] = want(sm->n_entries[d], n * 4);
+        o_epc[d] = want(sm->endpoint_counts[d], n * c->packed[d].erows.size() * 8);
+    }
+    const size_t o_st_scratch = want_sm && !ho->status ? slot(n * sizeof(b2r_string_status)) : 0;   // the post-pass reads the status
     need = align_up(need, 256);
     int rc;
     if ((rc = c->ws_cols.reserve(need))) return rc;
@@ -221,6 +234,15 @@ int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, co
     dout.masked_chars = (uint8_t*)dp(ho->masked_chars, o_mc); dout.masked_substr_ids = (uint8_t*)dp(ho->masked_substr_ids, o_ms);
     dout.status = (b2r_string_status*)dp(ho->status, o_st); dout.records = (b2r_substr_record*)dp(ho->records, o_rec);
     dout.compact_bytes = (uint8_t*)dp(ho->compact_bytes, o_cb);
+    if (want_sm) {
+        if (!ho->status) dout.status = (b2r_string_status*)(dv + o_st_scratch);
+        dsm.max_entries = sm->max_entries;
+        for (uint32_t d = 0; d < c->n_defs; d++) {
+            if (!string_mult_wanted(c, sm, d)) continue;
+            dsm.entries[d] = (b2r_row_count*)dp(sm->entries[d], o_ent[d]); dsm.n_entries[d] = (uint32_t*)dp(sm->n_entries[d], o_nent[d]);
+            dsm.endpoint_counts[d] = (uint32_t*)dp(sm->endpoint_counts[d], o_epc[d]);
+        }
+    }
     // up: offsets (rebased to the arena), bytes, and the caller's counters when they accumulate
     uint64_t* ho_offs = (uint64_t*)(hv + off_offs);
     const uint64_t shift = base & 15;                                     // keep the strings' alignment inside 16-byte vectors
@@ -233,12 +255,24 @@ int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, co
     }
     w_prep = wall_us();
     CUDA_TRY(cudaMemcpyAsync(dv, hv, up_bytes, cudaMemcpyHostToDevice, st));
+    for (uint32_t d = 0; d < c->n_defs; d++)
+        if (dsm.entries[d]) {
+            const size_t bytes = n * (size_t)sm->max_entries * sizeof(b2r_row_count);
+            memcpy(hv + o_ent[d], sm->entries[d], bytes);
+            CUDA_TRY(cudaMemcpyAsync(dv + o_ent[d], hv + o_ent[d], bytes, cudaMemcpyHostToDevice, st));
+            up_bytes += bytes;
+        }
     w_up = wall_us();
     dout.flags &= ~(uint32_t)B2R_OUT_SPARSE_D2H;                          // nothing to gain on one tile
     c->counters_copy = (BatchCounters*)(dv + off_cnt);
     rc = entry(c, dv + off_bytes, (const uint64_t*)(dv + off_offs), n, shift + nbytes, &dout, c->max_chars, st);
     c->counters_copy = nullptr;
     if (rc) return rc;
+    if (want_sm) {
+        void* states[B2R_MAX_DEFS] = {};
+        for (uint32_t d = 0; d < c->n_defs; d++) states[d] = c->last.def[d].states;   // the caller's column or the scratch one
+        if ((rc = string_mult_impl(c, dv + off_bytes, (const uint64_t*)(dv + off_offs), n, c->max_chars, states, rp, dout.status, &dsm, st, &c->last_launches))) return rc;
+    }
     CUDA_TRY(cudaMemcpyAsync(hv + off_mult, dv + off_mult, need - off_mult, cudaMemcpyDeviceToHost, st));
     w_enq = wall_us();
     CUDA_TRY(cudaStreamSynchronize(st));
@@ -273,7 +307,7 @@ struct DeviceEntry {
 const DeviceEntry BATCH_ENTRY = {match_batch_impl, false}, CHUNKED_ENTRY = {match_batch_chunked_impl, true};
 
 int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result,
-               const MultiHook* hook) {
+               const MultiHook* hook, const b2r_string_mult_outputs* sm = nullptr) {
     if (!c || !ho || (n && !h_offsets)) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
     if (c->device < 0) { set_error("this handle was created without a device (device = -1): no CPU fallback exists"); return B2R_ERR_CUDA; }
     int rc = check_outputs(c, ho, false);  // same pitches are used on the device; host pointer alignment is irrelevant
@@ -294,7 +328,7 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
     const uint64_t nbytes = total - base;
     const uint64_t rp = ho->row_pitch, bp = ho->bitmap_pitch;
     if (!hook && c->opt.small_path && n >= 1 && n <= 32 && n * (rp * (4 + 3 * c->n_defs) + 2 * bp * c->n_defs) + nbytes <= (8u << 20))
-        return host_batch_small(c, entry.run, h_bytes, h_offsets, n, ho, result);
+        return host_batch_small(c, entry.run, h_bytes, h_offsets, n, ho, sm, result);
 
     if ((rc = c->ws_bytes.reserve(align_up(nbytes + 16, 256)))) return rc;
     if ((rc = c->ws_offsets.reserve((n + 1) * 8))) return rc;
@@ -331,6 +365,17 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
     const size_t off_st = ho->status ? slot(n * sizeof(b2r_string_status)) : 0;
     const size_t off_rec = ho->records ? slot(n * (size_t)ho->max_records * sizeof(b2r_substr_record)) : 0;
     const size_t off_cb = ho->compact_bytes ? slot(n * (size_t)ho->compact_pitch) : 0;
+    // per-string counts (b2r_match_batch_host_mult): copied back per slice like the status
+    bool want_sm = false;
+    size_t off_ent[B2R_MAX_DEFS] = {}, off_nent[B2R_MAX_DEFS] = {}, off_epc[B2R_MAX_DEFS] = {};
+    for (uint32_t d = 0; d < c->n_defs; d++) {
+        if (!string_mult_wanted(c, sm, d)) continue;
+        want_sm = true;
+        off_ent[d] = sm->entries[d] ? slot(n * (size_t)sm->max_entries * sizeof(b2r_row_count)) : 0;
+        off_nent[d] = sm->n_entries[d] ? slot(n * 4) : 0;
+        off_epc[d] = sm->endpoint_counts[d] ? slot(n * c->packed[d].erows.size() * 8) : 0;
+    }
+    const size_t off_st_scratch = want_sm && !ho->status ? slot(n * sizeof(b2r_string_status)) : 0;   // the post-pass reads the status
     if ((rc = c->ws_cols.reserve(need + 256))) return rc;
     unsigned char* cb = (unsigned char*)c->ws_cols.p;
     auto bind = [&](void* host, size_t off, size_t bytes, size_t stride = 0, bool sp = false) -> void* {
@@ -364,6 +409,17 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
     dout.status = (b2r_string_status*)bind(ho->status, off_st, n * sizeof(b2r_string_status), sizeof(b2r_string_status));
     dout.records = (b2r_substr_record*)bind(ho->records, off_rec, n * (size_t)ho->max_records * sizeof(b2r_substr_record), (size_t)ho->max_records * sizeof(b2r_substr_record));
     dout.compact_bytes = (uint8_t*)bind(ho->compact_bytes, off_cb, n * (size_t)ho->compact_pitch, (size_t)ho->compact_pitch);
+    b2r_string_mult_outputs dsm{};
+    if (want_sm) {
+        if (!ho->status) dout.status = (b2r_string_status*)(cb + off_st_scratch);
+        dsm.max_entries = sm->max_entries;
+        for (uint32_t d = 0; d < c->n_defs; d++) {
+            const size_t es = (size_t)sm->max_entries * sizeof(b2r_row_count), ps = c->packed[d].erows.size() * 8;
+            dsm.entries[d] = (b2r_row_count*)bind(sm->entries[d], off_ent[d], n * es, es);
+            dsm.n_entries[d] = (uint32_t*)bind(sm->n_entries[d], off_nent[d], n * 4, 4);
+            dsm.endpoint_counts[d] = (uint32_t*)bind(sm->endpoint_counts[d], off_epc[d], n * ps, ps);
+        }
+    }
 
     // The batch is cut into slices of strings: the H2D copy of slice i+1 and the D2H copy of slice i-1 run on their own
     // streams while the kernels of slice i run (PCIe is full duplex; the copies are the end-to-end bottleneck).
@@ -515,6 +571,12 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
         slice_lo[i] = lo;
         const uint64_t b0 = n ? h_offsets[lo] : 0, b1 = n ? h_offsets[hi] : 0;
         if (b1 > b0) { CUDA_TRY(cudaMemcpyAsync(d_in + (b0 - base), h_bytes + b0, b1 - b0, cudaMemcpyHostToDevice, c->in_stream)); h2d += b1 - b0; }
+        for (uint32_t d = 0; d < c->n_defs && ni; d++)                  // entry slots the post-pass does not write keep the caller's values
+            if (dsm.entries[d]) {
+                const size_t es = (size_t)sm->max_entries * sizeof(b2r_row_count);
+                CUDA_TRY(cudaMemcpyAsync((unsigned char*)dsm.entries[d] + lo * es, (const unsigned char*)sm->entries[d] + lo * es, ni * es, cudaMemcpyHostToDevice, c->in_stream));
+                h2d += ni * es;
+            }
         CUDA_TRY(cudaEventRecord(c->ev_in[i], c->in_stream));
         CUDA_TRY(cudaStreamWaitEvent(st, c->ev_in[i], 0));
         b2r_outputs ds = dout;                                           // this slice's rows of every column
@@ -547,6 +609,17 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
         c->counters_copy = nullptr;
         c->sparse_zeroed = false;
         if (rc) return rc;
+        if (want_sm && ni) {
+            b2r_string_mult_outputs s = dsm;
+            void* states[B2R_MAX_DEFS] = {};
+            for (uint32_t d = 0; d < c->n_defs; d++) {
+                states[d] = c->last.def[d].states;                       // the caller's column or the scratch one, this slice's rows
+                if (s.entries[d]) s.entries[d] += lo * sm->max_entries;
+                if (s.n_entries[d]) s.n_entries[d] += lo;
+                if (s.endpoint_counts[d]) s.endpoint_counts[d] += lo * 2 * c->packed[d].erows.size();
+            }
+            if ((rc = string_mult_impl(c, d_bytes, d_offsets + lo, ni, c->max_chars, states, rp, ds.status, &s, st, &c->last_launches))) return rc;
+        }
         slice_params[i] = c->last;
         launches += c->last_launches;
         if (sparse && ni)
@@ -746,7 +819,8 @@ int multi_set_option(MultiState* m, const char* name, const char* value) {
 
 namespace {
 
-int multi_host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result) {
+int multi_host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result,
+                     const b2r_string_mult_outputs* sm = nullptr) {
     MultiState* m = c->multi;
     const int nd = (int)m->kids.size();
     if (!ho || (n && !h_offsets)) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
@@ -786,11 +860,20 @@ int multi_host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_b
             if (o.status) o.status += lo;
             if (o.records) o.records += lo * (size_t)ho->max_records;
             if (o.compact_bytes) o.compact_bytes += lo * (size_t)ho->compact_pitch;
+            b2r_string_mult_outputs s{};                                 // per-string counts: this device's strings, no exchange
+            if (sm) {
+                s = *sm;
+                for (uint32_t d = 0; d < kid->n_defs; d++) {
+                    if (s.entries[d]) s.entries[d] += lo * sm->max_entries;
+                    if (s.n_entries[d]) s.n_entries[d] += lo;
+                    if (s.endpoint_counts[d]) s.endpoint_counts[d] += lo * 2 * kid->packed[d].erows.size();
+                }
+            }
             MultiHook hook;
             hook.comm = m->comms[k]; hook.all_reduce = m->all_reduce; hook.error_string = m->error_string; hook.first = k == 0;
             memset(&res[k], 0, sizeof res[k]);
             static const uint64_t zero_off[1] = {0};
-            rcs[k] = host_batch(kid, entry, h_bytes, n ? h_offsets + lo : zero_off, hi - lo, &o, &res[k], &hook);
+            rcs[k] = host_batch(kid, entry, h_bytes, n ? h_offsets + lo : zero_off, hi - lo, &o, &res[k], &hook, sm ? &s : nullptr);
             if (rcs[k]) errs[k] = get_error();
         });
     for (auto& t : threads) t.join();
@@ -865,6 +948,36 @@ int b2r_match_batch_chunked_host(b2r_config* c, const uint8_t* h_bytes, const ui
     if (!c) { set_error("null config"); return B2R_ERR_INVALID_ARG; }
     if (c->multi) return multi_host_batch(c, CHUNKED_ENTRY, h_bytes, h_offsets, n, ho, result);
     return host_batch(c, CHUNKED_ENTRY, h_bytes, h_offsets, n, ho, result, nullptr);
+}
+
+}  // extern "C"
+
+namespace {
+
+int host_batch_mult(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
+                    const b2r_string_mult_outputs* sm, b2r_batch_status* result) {
+    // the arguments are checked first (the same answer on any handle), then the device
+    if (!c) { set_error("null config"); return B2R_ERR_INVALID_ARG; }
+    if (!ho || !sm) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
+    const int rc = check_string_mult(c, sm);
+    if (rc) return rc;
+    if (!c->multi && c->device < 0) { set_error("this handle was created without a device (device = -1): no CPU fallback exists"); return B2R_ERR_CUDA; }
+    if (c->multi) return multi_host_batch(c, entry, h_bytes, h_offsets, n, ho, result, sm);
+    return host_batch(c, entry, h_bytes, h_offsets, n, ho, result, nullptr, sm);
+}
+
+}  // namespace
+
+extern "C" {
+
+int b2r_match_batch_host_mult(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
+                              const b2r_string_mult_outputs* sm, b2r_batch_status* result) {
+    return host_batch_mult(c, BATCH_ENTRY, h_bytes, h_offsets, n, ho, sm, result);
+}
+
+int b2r_match_batch_chunked_host_mult(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
+                                      const b2r_string_mult_outputs* sm, b2r_batch_status* result) {
+    return host_batch_mult(c, CHUNKED_ENTRY, h_bytes, h_offsets, n, ho, sm, result);
 }
 
 int b2r_match_substrs(b2r_config* c, const uint8_t* characters, uint64_t len, const b2r_outputs* h_out, b2r_batch_status* result) {

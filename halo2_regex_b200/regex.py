@@ -149,6 +149,61 @@ class DeviceOutputs:
         return tot
 
 
+class StringMultOutputs:
+    """Per-string lookup multiplicities (include/b2r.h `b2r_string_mult_outputs`) as torch tensors: per def `entries[d]`
+    (n, max_entries, 2) int32 holding (row, count) pairs as u32, `n_entries[d]` (n,), `endpoint_counts[d]` (n, 2*E_d).
+    `device`: the handle's GPU by default (b2r_string_mult), "cpu" for the host entry points (`pin=True`: page-locked).
+    `max_entries` defaults to max_d min(M, T_d), which never truncates; `fill`: a byte pattern for every buffer."""
+
+    WANT = ("entries", "n_entries", "endpoint_counts")
+
+    def __init__(self, cfg, n, max_entries=None, device=None, want=WANT, fill=None, pin=False, max_chars_size=None):
+        import torch
+        self.cfg, self.n = cfg, int(n)
+        self.m = int(max_chars_size) if max_chars_size else cfg.max_chars_size
+        self.max_entries = int(max_entries) if max_entries is not None else max(min(self.m, t) for t in cfg.table_num_rows)
+        if device is None:
+            device = torch.device("cuda", cfg.device) if cfg.device >= 0 else "cpu"
+        dev = torch.device(device)
+        self.want = set(want)
+
+        def z(shape):
+            t = torch.empty(shape, dtype=torch.int32, device=dev, pin_memory=pin and dev.type == "cpu")
+            if fill is not None:
+                t.view(torch.uint8).fill_(fill)
+            return t
+
+        D = cfg.n_defs
+        self.entries = [z((self.n, self.max_entries, 2)) if "entries" in self.want else None for _ in range(D)]
+        self.n_entries = [z((self.n,)) if "n_entries" in self.want or "entries" in self.want else None for _ in range(D)]
+        self.endpoint_counts = [z((self.n, 2 * cfg.endpoint_num_rows[d])) if "endpoint_counts" in self.want else None for d in range(D)]
+
+    def struct(self):
+        s = _abi.StringMultStruct()
+        s.max_entries = self.max_entries
+        for d in range(self.cfg.n_defs):
+            for name in ("entries", "n_entries", "endpoint_counts"):
+                t = getattr(self, name)[d]
+                getattr(s, name)[d] = None if t is None else t.data_ptr()
+        return s
+
+    def to_host(self):
+        """A copy of every buffer in host memory."""
+        h = StringMultOutputs.__new__(StringMultOutputs)
+        h.cfg, h.n, h.m, h.max_entries, h.want = self.cfg, self.n, self.m, self.max_entries, set(self.want)
+        for name in ("entries", "n_entries", "endpoint_counts"):
+            setattr(h, name, [None if t is None else t.cpu() for t in getattr(self, name)])
+        return h
+
+    def dense(self, j, d):
+        """The T_d-long count vector of string j (uint64): the mult[d] of a one-string batch of that string."""
+        out = np.zeros(self.cfg.table_num_rows[d], dtype=np.uint64)
+        k = min(int(self.n_entries[d][j]), self.max_entries)
+        e = self.entries[d][j, :k].cpu().numpy().view(np.uint32)
+        out[e[:, 0]] = e[:, 1]
+        return out
+
+
 class RegexVerifyConfig:
     """reference src/lib.rs:97-113.  `configure` takes the two parameters that matter for witness generation
     (`max_chars_size`, `regex_defs`, src/lib.rs:126-131); `meta` / `gate` belong to the halo2 side and are ignored."""
@@ -255,6 +310,39 @@ class RegexVerifyConfig:
         if check:
             _raise(rc, res)
         return out, res
+
+    def match_batch_host_mult(self, data, offsets, out=None, sm=None, flags=0, check=True, sparse=False, reuse=False, max_entries=None, **kw):
+        """b2r_match_batch_host_mult: match_batch_host plus the per-string lookup multiplicities into `sm` (a host
+        StringMultOutputs, allocated here if not given).  Returns (out, sm, batch result)."""
+        return self._host_call_mult(lib.b2r_match_batch_host_mult, data, offsets, out, sm, flags, check, sparse, reuse, max_entries, kw)
+
+    def match_batch_chunked_host_mult(self, data, offsets, out=None, sm=None, flags=0, check=True, sparse=False, reuse=False, max_entries=None, **kw):
+        """b2r_match_batch_chunked_host_mult: match_batch_chunked_host plus the per-string lookup multiplicities."""
+        return self._host_call_mult(lib.b2r_match_batch_chunked_host_mult, data, offsets, out, sm, flags, check, sparse, reuse, max_entries, kw)
+
+    def _host_call_mult(self, fn, data, offsets, out, sm, flags, check, sparse, reuse, max_entries, kw):
+        n = len(offsets) - 1
+        if sm is None:
+            sm = StringMultOutputs(self, n, max_entries=max_entries, device="cpu")
+        s = sm.struct()
+        call = lambda h, b, o, n_, st, res: fn(h, b, o, n_, st, C.byref(s), res)  # noqa: E731
+        out, res = self._host_call(call, data, offsets, out, flags, check, sparse, reuse, kw)
+        return out, sm, res
+
+    def string_mult_device(self, d_bytes, d_offsets, out, sm=None, max_chars_size=0, stream=None, max_entries=None):
+        """b2r_string_mult: per-string lookup multiplicities from the state columns and status that an earlier
+        match_batch_device / match_batch_chunked_device / match_long_device call wrote into `out` (same bytes and offsets;
+        after match_long_device pass max_chars_size = len + 1 and offsets [0, len]).  Asynchronous on `stream`.  Returns `sm`."""
+        import torch
+        if stream is None:
+            stream = torch.cuda.current_stream(d_bytes.device)
+        n = d_offsets.numel() - 1
+        if sm is None:
+            sm = StringMultOutputs(self, n, max_entries=max_entries, device=d_bytes.device, max_chars_size=max_chars_size or None)
+        rc = lib.b2r_string_mult(self._h, d_bytes.data_ptr(), d_offsets.data_ptr(), n, d_bytes.numel(), int(max_chars_size),
+                                 C.byref(out.struct()), C.byref(sm.struct()), stream.cuda_stream)
+        _raise(rc)
+        return sm
 
     def match_strings(self, strings, **kw):
         data = np.frombuffer(b"".join(strings), dtype=np.uint8) if strings else np.zeros(0, np.uint8)

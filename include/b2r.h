@@ -131,8 +131,8 @@ uint32_t b2r_config_num_devices(const b2r_config*);
  *   stagger_ns   start offset between the warps of a walk CTA (-1: default)
  *   slices, host_threads, small_path, sparse_cap, sparse_direct, trace_host   host entry points (b2r_match_batch_host)
  *   hist_cache_log2, spread_fill, long_fused, debug, host_debug               kernel tuning / timing experiments
- *   chunked_max_maps   b2r_match_batch_chunked: bytes of chunk transition vectors per pass (0: the default 1 GiB); small
- *                      values force many passes */
+ *   chunked_max_maps   b2r_match_batch_chunked: bytes of chunk transition vectors per pass (0: the default 1 GiB); b2r_string_mult:
+ *                      bytes of per-string counters per pass (0: the default 256 MiB); small values force many passes */
 int b2r_config_set_option(b2r_config*, const char* name, const char* value);
 
 /* Page-locked host memory for the buffers handed to the host-pointer entry points (a copy into pageable memory cannot overlap
@@ -299,6 +299,62 @@ int b2r_match_long(b2r_config* cfg, const uint8_t* d_bytes, uint64_t len, const 
  * the string is copied up, the M = len+1 rows of every requested column are copied back; row_pitch >= M. */
 int b2r_match_long_host(b2r_config* cfg, const uint8_t* h_bytes, uint64_t len, const b2r_outputs* h_out,
                         b2r_batch_status* result);
+
+/* ---- per-string lookup multiplicities ---------------------------------------------------------------------------------------------
+ * mult / endpoint_mult of b2r_outputs are sums over every string of a call: the multiplicity column of ONE lookup argument over
+ * the whole batch.  A prover that makes one proof per string (the reference: one match_substrs per synthesize pass,
+ * src/lib.rs:311-318) needs them per string.  b2r_string_mult computes them on the device from the state columns an earlier call
+ * wrote; the _mult host entry points run the same post-pass inside the host pipeline.
+ *
+ * Contract:
+ *   - Definition.  For every string without B2R_ST_INVALID_TRANSITION or B2R_ST_TOO_LONG, the counts of string j and def d are
+ *     exactly the mult[d] and endpoint_mult[d] that a one-string b2r_match_batch of string j writes, on the same handle with the
+ *     same M.  A stored entry is a (row, count) with count > 0, rows ascending (rows of b2r_table_rows).  Row 0 carries M - len,
+ *     so sum(count) = M, and each half of endpoint_counts sums to M.
+ *   - Flagged strings.  A string flagged invalid or too long gets n_entries = 0 and all-zero endpoint counts; its entry slots are
+ *     left untouched (the reference panics on such a string and counts nothing).  So over all strings of a call, sum_j of the
+ *     per-string counts equals the batch mult[d] / endpoint_mult[d] of the same call.  The post-pass applies the too-long rule to
+ *     its own max_chars_size as well: a string with len > M - 1 for the M passed here (e.g. the handle's M after a b2r_match_long
+ *     of a longer string) is treated like a flagged one, whatever its status says.
+ *   - The state columns and status must be those the match call wrote for the same bytes and offsets; other contents give
+ *     unspecified counts (the call still completes).
+ *   - Truncation.  n_entries[j] is the true number of distinct rows; only the first max_entries (the lowest rows) are stored, and
+ *     the slots after n_entries are left untouched.  max_entries >= min(M, T_d) never truncates.
+ *   - Errors (nothing is enqueued): B2R_ERR_INVALID_ARG for a non-NULL entries[d] with a NULL n_entries[d], max_entries == 0 with
+ *     entries set, and (device entry only) a NULL status or a NULL states[d] of a def whose counts are asked for;
+ *     B2R_ERR_ALIGNMENT for entries not 8-byte aligned or n_entries / endpoint_counts not 4-byte aligned; B2R_ERR_CUDA on a handle
+ *     created with device = -1; B2R_ERR_INVALID_ARG for b2r_string_mult on a multi-device handle (b2r_config_new_multi: the device
+ *     entry takes pointers of one device; the host entries split the strings over the devices).
+ *   - b2r_last_launch_count counts the post-pass kernels (one per pass of strings, plus one compaction per pass when M - 1 > 4096).
+ * Cost: the post-pass reads the bytes and the state columns once and writes 8 bytes per stored entry.  A string longer than 4096
+ * bytes is counted in pieces into a device workspace of (T_d + 2 E_d) u32 per string and def, in passes of at most 256 MiB of it
+ * (chunked_max_maps, when set, bounds it instead), which the handle keeps. */
+typedef struct b2r_row_count {
+    uint32_t row;
+    uint32_t count;
+} b2r_row_count; /* 8 bytes */
+
+typedef struct b2r_string_mult_outputs {
+    uint32_t max_entries;                     /* entries reserved per string and def */
+    uint32_t reserved;
+    b2r_row_count* entries[B2R_MAX_DEFS];     /* N * max_entries, string j at j * max_entries, rows ascending; or NULL */
+    uint32_t* n_entries[B2R_MAX_DEFS];        /* N: number of distinct rows of string j (may exceed max_entries); or NULL */
+    uint32_t* endpoint_counts[B2R_MAX_DEFS];  /* N * 2*E_d (E_d = b2r_endpoint_num_rows), dense, halves as in endpoint_mult; or NULL */
+} b2r_string_mult_outputs;
+
+/* Device post-pass over the columns that an earlier b2r_match_batch / b2r_match_batch_chunked / b2r_match_long call on the same
+ * bytes and offsets wrote: reads d_out->states[d], row_pitch and status.  Asynchronous on cuda_stream.
+ * max_chars_size 0 = the handle's M (after b2r_match_long: pass len + 1, and offsets {0, len}). */
+int b2r_string_mult(b2r_config* cfg, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n_strings, uint64_t total_bytes,
+                    uint64_t max_chars_size, const b2r_outputs* d_out, const b2r_string_mult_outputs* d_sm, void* cuda_stream);
+
+/* b2r_match_batch_host / b2r_match_batch_chunked_host plus the per-string counts (host pointers), copied back with each slice.
+ * h_out->states and h_out->status may be NULL: the library then uses its own scratch columns.  Every column, status, record and
+ * counter is what the call without _mult writes; the entry slots the post-pass does not write keep what the caller had in them. */
+int b2r_match_batch_host_mult(b2r_config* cfg, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n_strings,
+                              const b2r_outputs* h_out, const b2r_string_mult_outputs* h_sm, b2r_batch_status* result);
+int b2r_match_batch_chunked_host_mult(b2r_config* cfg, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n_strings,
+                                      const b2r_outputs* h_out, const b2r_string_mult_outputs* h_sm, b2r_batch_status* result);
 
 /* ---- the step after the path: witness columns as field elements (SURVEY 8(f) rank 1) ------------------------------------------
  * The reference places every value of the path in a cell as Value::known(F::from(x as u64)) (src/lib.rs:342-347, 388-418), with
