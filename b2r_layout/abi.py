@@ -104,6 +104,16 @@ class StringMultStruct(C.Structure):
     ]
 
 
+class StringMultPackedStruct(C.Structure):
+    """b2r_string_mult_packed_outputs"""
+    _fields_ = [
+        ("capacity", C.c_uint64),
+        ("entries", C.c_void_p * B2R_MAX_DEFS),
+        ("row_start", C.c_void_p * B2R_MAX_DEFS),
+        ("endpoint_counts", C.c_void_p * B2R_MAX_DEFS),
+    ]
+
+
 assert C.sizeof(StringStatus) == 32
 assert C.sizeof(RowCount) == 8
 assert C.sizeof(SubstrRecord) == 16

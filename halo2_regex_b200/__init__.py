@@ -8,7 +8,7 @@ from ._ffi import LIB_PATH, SYMBOLS, last_error, lib  # noqa: F401
 from .buffers import HostOutputs, PinnedAllocator, compare_outputs  # noqa: F401
 from .defs import AllstrRegexDef, RegexDefs, RegexParseError, SubstrRegexDef  # noqa: F401
 from .regex import (AssignedRegexResult, DeviceOutputs, InvalidTransitionError, RegexVerifyConfig,  # noqa: F401
-                    StringMultOutputs, StringTooLongError)
+                    StringMultOutputs, StringMultPacked, StringTooLongError)
 
 from . import vrm  # noqa: F401,E402  (host-side definition compiler: regex JSON -> lookup text files)
 

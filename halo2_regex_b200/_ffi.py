@@ -27,6 +27,7 @@ b2r_config_set_timing b2r_last_kernel_ms b2r_last_stage_ms b2r_last_plan
 b2r_config_new_multi b2r_config_num_devices b2r_config_set_option b2r_host_alloc b2r_host_free b2r_host_register b2r_host_unregister
 b2r_last_host_bytes b2r_column_to_fr
 b2r_string_mult b2r_match_batch_host_mult b2r_match_batch_chunked_host_mult
+b2r_string_mult_packed b2r_match_batch_host_mult_packed b2r_match_batch_chunked_host_mult_packed
 """.split()
 
 
@@ -101,6 +102,11 @@ def _load():
     sig("b2r_string_mult", i32, vp, vp, vp, u64, u64, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.StringMultStruct), vp)
     sig("b2r_match_batch_host_mult", i32, vp, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.StringMultStruct), C.POINTER(_abi.BatchStatus))
     sig("b2r_match_batch_chunked_host_mult", i32, vp, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.StringMultStruct),
+        C.POINTER(_abi.BatchStatus))
+    sig("b2r_string_mult_packed", i32, vp, vp, vp, u64, u64, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.StringMultPackedStruct), vp)
+    sig("b2r_match_batch_host_mult_packed", i32, vp, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.StringMultPackedStruct),
+        C.POINTER(_abi.BatchStatus))
+    sig("b2r_match_batch_chunked_host_mult_packed", i32, vp, vp, vp, u64, C.POINTER(_abi.Outputs), C.POINTER(_abi.StringMultPackedStruct),
         C.POINTER(_abi.BatchStatus))
     return L
 

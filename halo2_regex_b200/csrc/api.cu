@@ -420,10 +420,10 @@ void b2r_config_free(b2r_config* c) {
     if (c->device >= 0) {
         DeviceGuard g(c->device);
         cudaFree(c->tables); cudaFree(c->scratch); cudaFree(c->d_batch_status);
-        c->ws_fmask.release(); c->ws_long.release(); c->ws_smult.release();
+        c->ws_fmask.release(); c->ws_long.release(); c->ws_smult.release(); c->ws_smpk.release();
         for (auto& b : c->ws_states) b.release();
         c->ws_bytes.release(); c->ws_offsets.release(); c->ws_cols.release(); c->ws_sparse.release(); c->ws_sparse_arena.release();
-        c->pin_sparse[0].release(); c->pin_sparse[1].release(); c->pin_small.release();
+        c->pin_sparse[0].release(); c->pin_sparse[1].release(); c->pin_small.release(); c->pin_pk.release();
         if (c->host_stream) cudaStreamDestroy(c->host_stream);
         if (c->in_stream) cudaStreamDestroy(c->in_stream);
         if (c->out_stream) cudaStreamDestroy(c->out_stream);

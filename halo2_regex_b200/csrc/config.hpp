@@ -156,6 +156,7 @@ struct b2r_config {
     b2r::DevBuf ws_long;                   // long-string path: chunk offsets, transition-vector tree, entry states, flag summary
     b2r::DevBuf ws_states[B2R_MAX_DEFS];   // state column of a def the caller did not ask for (emit reads it)
     b2r::DevBuf ws_smult;                  // per-string counters of strings longer than one string_mult segment (string_mult.cu)
+    b2r::DevBuf ws_smpk;                   // packed per-string counts: running totals, list lengths and slots of one pass (string_mult.cu)
     b2r::WalkParams last = {};
     bool have_last = false;
     uint32_t last_launches = 0;
@@ -164,6 +165,7 @@ struct b2r_config {
     // staging for the host-pointer entry points
     b2r::DevBuf ws_bytes, ws_offsets, ws_cols, ws_sparse, ws_sparse_arena;
     b2r::PinBuf pin_sparse[2], pin_small;
+    b2r::PinBuf pin_pk;                    // packed per-string counts: slice totals and slice-relative row_start values on their way back
     cudaStream_t host_stream = nullptr;
     cudaStream_t in_stream = nullptr, out_stream = nullptr;   // host entry point: H2D / D2H copies overlapping the kernels
     cudaStream_t pay_stream = nullptr;                        // sparse D2H mode: the compacted sectors of a slice
@@ -203,6 +205,15 @@ int check_string_mult(const b2r_config* c, const b2r_string_mult_outputs* sm);
 bool string_mult_wanted(const b2r_config* c, const b2r_string_mult_outputs* sm, uint32_t d);
 int string_mult_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t max_chars, void* const* states,
                      uint64_t row_pitch, const b2r_string_status* status, const b2r_string_mult_outputs* sm, cudaStream_t st, uint32_t* launches);
+// the packed layout: argument checks, the workspace of a call over at most n strings (reserved before a host pipeline enqueues
+// its first slice), and the post-pass itself.  row_start is written relative to the call's first string; with host_total
+// (pinned, [n_defs]) the call's total per def is also stored there by a kernel, readable once the stream has passed the call.
+bool string_mult_packed_wanted(const b2r_config* c, const b2r_string_mult_packed_outputs* pk, uint32_t d);
+int check_string_mult_packed(const b2r_config* c, const b2r_string_mult_packed_outputs* pk);
+int string_mult_packed_reserve(b2r_config* c, uint64_t n, uint64_t max_chars, const b2r_string_mult_packed_outputs* pk);
+int string_mult_packed_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t max_chars, void* const* states,
+                            uint64_t row_pitch, const b2r_string_status* status, const b2r_string_mult_packed_outputs* pk, uint64_t* host_total,
+                            cudaStream_t st, uint32_t* launches);
 // host.cu
 void multi_free(MultiState* m);
 int multi_set_option(MultiState* m, const char* name, const char* value);

@@ -15,7 +15,10 @@
 #include <nccl.h>   // types and prototypes only: the library is dlopen'ed (libb2r.so does not link against NCCL)
 
 #include <algorithm>
+#include <array>
 #include <chrono>
+#include <condition_variable>
+#include <mutex>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -144,6 +147,33 @@ struct MultiHook {
     ncclResult_t (*all_reduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
     const char* (*error_string)(ncclResult_t) = nullptr;
     bool first = true;                 // this device uploads the caller's counters (accumulate) and copies the result back
+    // packed per-string counts: the entries of device k start where those of devices < k end
+    struct PkChain* chain = nullptr;
+    int index = 0;
+    bool last = true;                  // this device writes row_start[N]
+};
+
+// The totals a multi-device packed call's devices publish in device order (device k waits for devices < k before it issues its
+// entry copies).  A device publishes exactly once, also when its call fails, so that no other device waits forever.
+struct PkChain {
+    std::mutex m;
+    std::condition_variable cv;
+    std::vector<char> done;
+    std::vector<std::array<uint64_t, B2R_MAX_DEFS>> total;
+    explicit PkChain(int n) : done(n, 0), total(n) {}
+    void publish(int k, const uint64_t* t) {
+        { std::lock_guard<std::mutex> l(m); if (done[k]) return; for (int d = 0; d < B2R_MAX_DEFS; d++) total[k][d] = t[d]; done[k] = 1; }
+        cv.notify_all();
+    }
+    void base(int k, uint64_t* b) {
+        std::unique_lock<std::mutex> l(m);
+        cv.wait(l, [&] { for (int q = 0; q < k; q++) if (!done[q]) return false; return true; });
+        for (int d = 0; d < B2R_MAX_DEFS; d++) { b[d] = 0; for (int q = 0; q < k; q++) b[d] += total[q][d]; }
+    }
+};
+struct PkPublishOnExit {
+    const MultiHook* hook;
+    ~PkPublishOnExit() { if (hook && hook->chain) { const uint64_t z[B2R_MAX_DEFS] = {}; hook->chain->publish(hook->index, z); } }
 };
 
 unsigned default_host_threads() {
@@ -169,12 +199,29 @@ bool is_pinned(const void* h) {
     return a.type == cudaMemoryTypeHost;
 }
 
+// ---- packed per-string counts: what a slice's lists take, and how many of its entries are stored ----------------------------------
+// slots per string of the packed post-pass (string_mult.cu): no list is longer
+uint64_t pk_pitch(const b2r_config* c, uint64_t M) {
+    uint64_t w = 1;
+    for (uint32_t d = 0; d < c->n_defs; d++) w = std::max<uint64_t>(w, std::min<uint64_t>(M, c->packed[d].rows.size()));
+    return w;
+}
+
+// The entries of ni strings whose lists start at `base` in the caller's area and which are stored under `cap`: the lists of a prefix
+// of them (row_start does not decrease), none in part.  rel[k - 1] = row_start[k] - base for 1 <= k <= ni, so rel[ni - 1] is the total.
+uint64_t pk_stored(uint64_t base, uint64_t cap, const uint64_t* rel, uint64_t ni) {
+    if (!ni || base >= cap) return 0;
+    if (base + rel[ni - 1] <= cap) return rel[ni - 1];
+    const uint64_t* p = std::upper_bound(rel, rel + ni, cap - base);    // the first list end beyond the capacity
+    return p == rel ? 0 : p[-1];
+}
+
 // ---- small batches: one tile, one copy each way ------------------------------------------------------------------------------
 // Everything the call needs lives in ONE device arena (ws_cols) mirrored by ONE pinned host arena (pin_small):
 //   [offsets (n+1) u64 | input bytes | multiplicity block | BatchCounters copy | every requested column]
 // the first three parts go up in one copy, everything from the multiplicity block on comes back in one copy.
 int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
-                     const b2r_string_mult_outputs* sm, b2r_batch_status* result) {
+                     const b2r_string_mult_outputs* sm, const b2r_string_mult_packed_outputs* pk, b2r_batch_status* result) {
     cudaStream_t st = c->host_stream;
     const bool trace = c->opt.trace_host;
     const auto wall0 = std::chrono::steady_clock::now();
@@ -218,7 +265,21 @@ int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, co
         o_nent[d] = want(sm->n_entries[d], n * 4);
         o_epc[d] = want(sm->endpoint_counts[d], n * c->packed[d].erows.size() * 8);
     }
-    const size_t o_st_scratch = want_sm && !ho->status ? slot(n * sizeof(b2r_string_status)) : 0;   // the post-pass reads the status
+    bool want_pk = false;
+    for (uint32_t d = 0; d < c->n_defs; d++) want_pk = want_pk || string_mult_packed_wanted(c, pk, d);
+    const size_t o_st_scratch = (want_sm || want_pk) && !ho->status ? slot(n * sizeof(b2r_string_status)) : 0;   // the post-pass reads the status
+    need = align_up(need, 256);
+    // packed per-string counts (b2r_match_batch_host_mult_packed): after the arena's one copy, each part copied back exactly —
+    // row_start[1..n] (row_start[0] is 0) and the endpoint counts; the pack kernel stores the entries straight into the pinned
+    // arena (one slice: the capacity rule is the caller's), so only stored entries cross
+    const size_t pk_begin = need;
+    size_t o_pk_rs[B2R_MAX_DEFS] = {}, o_pk_ep[B2R_MAX_DEFS] = {}, o_pk_ent[B2R_MAX_DEFS] = {};
+    const uint64_t pk_cap = want_pk ? std::min<uint64_t>(pk->capacity, n * pk_pitch(c, c->max_chars)) : 0;   // n * pitch: every list fits
+    for (uint32_t d = 0; d < c->n_defs && want_pk; d++) {
+        if (pk->row_start[d]) o_pk_rs[d] = slot((n + 1) * 8, 8);
+        if (pk->endpoint_counts[d]) o_pk_ep[d] = slot(n * c->packed[d].erows.size() * 8, 8);
+        if (pk->row_start[d] && pk->entries[d] && pk_cap) o_pk_ent[d] = slot(pk_cap * sizeof(b2r_row_count), 8);
+    }
     need = align_up(need, 256);
     int rc;
     if ((rc = c->ws_cols.reserve(need))) return rc;
@@ -234,8 +295,8 @@ int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, co
     dout.masked_chars = (uint8_t*)dp(ho->masked_chars, o_mc); dout.masked_substr_ids = (uint8_t*)dp(ho->masked_substr_ids, o_ms);
     dout.status = (b2r_string_status*)dp(ho->status, o_st); dout.records = (b2r_substr_record*)dp(ho->records, o_rec);
     dout.compact_bytes = (uint8_t*)dp(ho->compact_bytes, o_cb);
+    if ((want_sm || want_pk) && !ho->status) dout.status = (b2r_string_status*)(dv + o_st_scratch);
     if (want_sm) {
-        if (!ho->status) dout.status = (b2r_string_status*)(dv + o_st_scratch);
         dsm.max_entries = sm->max_entries;
         for (uint32_t d = 0; d < c->n_defs; d++) {
             if (!string_mult_wanted(c, sm, d)) continue;
@@ -273,15 +334,45 @@ int host_batch_small(b2r_config* c, BatchEntry entry, const uint8_t* h_bytes, co
         for (uint32_t d = 0; d < c->n_defs; d++) states[d] = c->last.def[d].states;   // the caller's column or the scratch one
         if ((rc = string_mult_impl(c, dv + off_bytes, (const uint64_t*)(dv + off_offs), n, c->max_chars, states, rp, dout.status, &dsm, st, &c->last_launches))) return rc;
     }
-    CUDA_TRY(cudaMemcpyAsync(hv + off_mult, dv + off_mult, need - off_mult, cudaMemcpyDeviceToHost, st));
+    uint64_t pk_d2h = 0;
+    if (want_pk) {
+        b2r_string_mult_packed_outputs dpk{};
+        dpk.capacity = pk_cap;
+        void* states[B2R_MAX_DEFS] = {};
+        for (uint32_t d = 0; d < c->n_defs; d++) {
+            states[d] = c->last.def[d].states;
+            if (pk->row_start[d]) dpk.row_start[d] = (uint64_t*)(dv + o_pk_rs[d]);
+            if (pk->endpoint_counts[d]) dpk.endpoint_counts[d] = (uint32_t*)(dv + o_pk_ep[d]);
+            if (o_pk_ent[d]) dpk.entries[d] = (b2r_row_count*)(hv + o_pk_ent[d]);   // mapped pinned memory: the kernel stores across PCIe
+        }
+        if ((rc = string_mult_packed_impl(c, dv + off_bytes, (const uint64_t*)(dv + off_offs), n, c->max_chars, states, rp, dout.status, &dpk, nullptr, st,
+                                          &c->last_launches))) return rc;
+    }
+    CUDA_TRY(cudaMemcpyAsync(hv + off_mult, dv + off_mult, pk_begin - off_mult, cudaMemcpyDeviceToHost, st));
+    for (uint32_t d = 0; d < c->n_defs && want_pk; d++) {
+        if (pk->row_start[d]) { CUDA_TRY(cudaMemcpyAsync(hv + o_pk_rs[d] + 8, dv + o_pk_rs[d] + 8, n * 8, cudaMemcpyDeviceToHost, st)); pk_d2h += n * 8; }
+        const size_t eb = n * c->packed[d].erows.size() * 8;
+        if (pk->endpoint_counts[d]) { CUDA_TRY(cudaMemcpyAsync(hv + o_pk_ep[d], dv + o_pk_ep[d], eb, cudaMemcpyDeviceToHost, st)); pk_d2h += eb; }
+    }
     w_enq = wall_us();
     CUDA_TRY(cudaStreamSynchronize(st));
     w_sync = wall_us();
     for (const Part& p : parts) memcpy(p.host, hv + p.off, p.bytes);
+    for (uint32_t d = 0; d < c->n_defs && want_pk; d++) {
+        if (pk->endpoint_counts[d]) memcpy(pk->endpoint_counts[d], hv + o_pk_ep[d], n * c->packed[d].erows.size() * 8);
+        if (!pk->row_start[d]) continue;
+        uint64_t* rs = (uint64_t*)(hv + o_pk_rs[d]);
+        rs[0] = 0;
+        memcpy(pk->row_start[d], rs, (n + 1) * 8);
+        if (!o_pk_ent[d]) continue;
+        const uint64_t stored = pk_stored(0, pk->capacity, rs + 1, n);
+        if (stored) memcpy(pk->entries[d], hv + o_pk_ent[d], stored * sizeof(b2r_row_count));
+        pk_d2h += stored * sizeof(b2r_row_count);
+    }
     if (trace)
         fprintf(stderr, "[b2r] small batch (%llu strings): staged %.1f us, H2D issued %.1f, kernels + D2H issued %.1f, device done %.1f, copied out %.1f\n", (unsigned long long)n, w_prep,
                 w_up, w_enq, w_sync, wall_us());
-    c->last_h2d_bytes = up_bytes; c->last_d2h_bytes = need - off_mult;
+    c->last_h2d_bytes = up_bytes; c->last_d2h_bytes = pk_begin - off_mult + pk_d2h;
     const BatchCounters* hc = (const BatchCounters*)(hv + off_cnt);
     b2r_batch_status r;
     memset(&r, 0, sizeof r);
@@ -307,7 +398,8 @@ struct DeviceEntry {
 const DeviceEntry BATCH_ENTRY = {match_batch_impl, false}, CHUNKED_ENTRY = {match_batch_chunked_impl, true};
 
 int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result,
-               const MultiHook* hook, const b2r_string_mult_outputs* sm = nullptr) {
+               const MultiHook* hook, const b2r_string_mult_outputs* sm = nullptr, const b2r_string_mult_packed_outputs* pk = nullptr) {
+    PkPublishOnExit publish_on_exit{hook};
     if (!c || !ho || (n && !h_offsets)) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
     if (c->device < 0) { set_error("this handle was created without a device (device = -1): no CPU fallback exists"); return B2R_ERR_CUDA; }
     int rc = check_outputs(c, ho, false);  // same pitches are used on the device; host pointer alignment is irrelevant
@@ -328,7 +420,7 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
     const uint64_t nbytes = total - base;
     const uint64_t rp = ho->row_pitch, bp = ho->bitmap_pitch;
     if (!hook && c->opt.small_path && n >= 1 && n <= 32 && n * (rp * (4 + 3 * c->n_defs) + 2 * bp * c->n_defs) + nbytes <= (8u << 20))
-        return host_batch_small(c, entry.run, h_bytes, h_offsets, n, ho, sm, result);
+        return host_batch_small(c, entry.run, h_bytes, h_offsets, n, ho, sm, pk, result);
 
     if ((rc = c->ws_bytes.reserve(align_up(nbytes + 16, 256)))) return rc;
     if ((rc = c->ws_offsets.reserve((n + 1) * 8))) return rc;
@@ -375,7 +467,18 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
         off_nent[d] = sm->n_entries[d] ? slot(n * 4) : 0;
         off_epc[d] = sm->endpoint_counts[d] ? slot(n * c->packed[d].erows.size() * 8) : 0;
     }
-    const size_t off_st_scratch = want_sm && !ho->status ? slot(n * sizeof(b2r_string_status)) : 0;   // the post-pass reads the status
+    // packed per-string counts (b2r_match_batch_host_mult_packed): the endpoint counts are copied back per slice like the status;
+    // each slice packs its lists into its own staging area (lo * pitch on) with row_start relative to the slice (at lo + i)
+    bool want_pk = false;
+    for (uint32_t d = 0; d < c->n_defs; d++) want_pk = want_pk || string_mult_packed_wanted(c, pk, d);
+    const uint64_t pkw = want_pk ? pk_pitch(c, c->max_chars) : 0;
+    size_t off_pk_ep[B2R_MAX_DEFS] = {}, off_pk_rs[B2R_MAX_DEFS] = {}, off_pk_ent[B2R_MAX_DEFS] = {};
+    for (uint32_t d = 0; d < c->n_defs && want_pk; d++) {
+        off_pk_ep[d] = pk->endpoint_counts[d] ? slot(n * c->packed[d].erows.size() * 8) : 0;
+        off_pk_rs[d] = pk->row_start[d] ? slot((n + b2r_config::MAX_SLICES + 1) * 8) : 0;
+        off_pk_ent[d] = pk->row_start[d] && pk->entries[d] && pk->capacity ? slot(n * pkw * sizeof(b2r_row_count)) : 0;
+    }
+    const size_t off_st_scratch = (want_sm || want_pk) && !ho->status ? slot(n * sizeof(b2r_string_status)) : 0;   // the post-pass reads the status
     if ((rc = c->ws_cols.reserve(need + 256))) return rc;
     unsigned char* cb = (unsigned char*)c->ws_cols.p;
     auto bind = [&](void* host, size_t off, size_t bytes, size_t stride = 0, bool sp = false) -> void* {
@@ -410,8 +513,15 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
     dout.records = (b2r_substr_record*)bind(ho->records, off_rec, n * (size_t)ho->max_records * sizeof(b2r_substr_record), (size_t)ho->max_records * sizeof(b2r_substr_record));
     dout.compact_bytes = (uint8_t*)bind(ho->compact_bytes, off_cb, n * (size_t)ho->compact_pitch, (size_t)ho->compact_pitch);
     b2r_string_mult_outputs dsm{};
+    if ((want_sm || want_pk) && !ho->status) dout.status = (b2r_string_status*)(cb + off_st_scratch);
+    b2r_string_mult_packed_outputs dpk{};
+    for (uint32_t d = 0; d < c->n_defs && want_pk; d++) {
+        const size_t ps = c->packed[d].erows.size() * 8;
+        dpk.endpoint_counts[d] = (uint32_t*)bind(pk->endpoint_counts[d], off_pk_ep[d], n * ps, ps);
+        if (pk->row_start[d]) dpk.row_start[d] = (uint64_t*)(cb + off_pk_rs[d]);
+        if (off_pk_ent[d]) dpk.entries[d] = (b2r_row_count*)(cb + off_pk_ent[d]);
+    }
     if (want_sm) {
-        if (!ho->status) dout.status = (b2r_string_status*)(cb + off_st_scratch);
         dsm.max_entries = sm->max_entries;
         for (uint32_t d = 0; d < c->n_defs; d++) {
             const size_t es = (size_t)sm->max_entries * sizeof(b2r_row_count), ps = c->packed[d].erows.size() * 8;
@@ -467,6 +577,20 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
         if ((rc = chunked_reserve(c, widest, &dout, c->max_chars))) return rc;
     }
     auto cut = [&](int k) { return cuts[k]; };
+    // packed counts: the post-pass workspaces, sized for the widest slice before anything is enqueued; pinned: the totals the scan
+    // kernel publishes per slice and def, then per def the slice-relative row_start values that come back
+    uint64_t* pk_tot = nullptr;
+    uint64_t* pk_rel[B2R_MAX_DEFS] = {};
+    if (want_pk) {
+        uint64_t widest = 0;
+        for (int i = 0; i < n_slices; i++) widest = std::max(widest, cut(i + 1) - cut(i));
+        b2r_string_mult_packed_outputs shape = dpk;
+        shape.capacity = widest * pkw;
+        if ((rc = string_mult_packed_reserve(c, widest, c->max_chars, &shape))) return rc;
+        if ((rc = c->pin_pk.reserve(((size_t)b2r_config::MAX_SLICES * B2R_MAX_DEFS + (size_t)c->n_defs * (n + 1)) * 8))) return rc;
+        pk_tot = (uint64_t*)c->pin_pk.p;
+        for (uint32_t d = 0; d < c->n_defs; d++) pk_rel[d] = pk_tot + b2r_config::MAX_SLICES * B2R_MAX_DEFS + d * (n + 1);
+    }
 
     // ---- sparse mode: compaction arenas (device + pinned mirror) and the host threads ---------------------------------------------
     std::vector<const Copy*> scols;
@@ -620,6 +744,19 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
             }
             if ((rc = string_mult_impl(c, d_bytes, d_offsets + lo, ni, c->max_chars, states, rp, ds.status, &s, st, &c->last_launches))) return rc;
         }
+        if (want_pk && ni) {
+            b2r_string_mult_packed_outputs s{};
+            s.capacity = ni * pkw;                                        // the slice's staging holds every list: the caller's capacity is applied below
+            void* states[B2R_MAX_DEFS] = {};
+            for (uint32_t d = 0; d < c->n_defs; d++) {
+                states[d] = c->last.def[d].states;
+                if (dpk.row_start[d]) s.row_start[d] = dpk.row_start[d] + lo + i;
+                if (dpk.entries[d]) s.entries[d] = dpk.entries[d] + lo * pkw;
+                if (dpk.endpoint_counts[d]) s.endpoint_counts[d] = dpk.endpoint_counts[d] + lo * 2 * c->packed[d].erows.size();
+            }
+            if ((rc = string_mult_packed_impl(c, d_bytes, d_offsets + lo, ni, c->max_chars, states, rp, ds.status, &s, pk_tot + i * B2R_MAX_DEFS, st,
+                                              &c->last_launches))) return rc;
+        }
         slice_params[i] = c->last;
         launches += c->last_launches;
         if (sparse && ni)
@@ -747,6 +884,42 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
         memo.arena = arena;
         memo.valid = true;
     }
+    // ---- packed counts: slice i's total is in pinned memory when ev_done[i] fires; its stored entries go to the running offset ------
+    uint64_t pk_base[B2R_MAX_DEFS] = {};
+    if (want_pk) {
+        uint64_t mine[B2R_MAX_DEFS] = {};
+        for (int i = 0; i < n_slices; i++) {
+            if (cut(i + 1) == cut(i)) continue;
+            CUDA_TRY(cudaEventSynchronize(c->ev_done[i]));
+            for (uint32_t d = 0; d < c->n_defs; d++) if (dpk.row_start[d]) mine[d] += pk_tot[i * B2R_MAX_DEFS + d];
+        }
+        if (hook && hook->chain) { hook->chain->publish(hook->index, mine); hook->chain->base(hook->index, pk_base); }
+        for (uint32_t d = 0; d < c->n_defs; d++) {
+            if (!dpk.row_start[d]) continue;
+            uint64_t run = pk_base[d];
+            for (int i = 0; i < n_slices; i++) {
+                const uint64_t lo = cut(i), ni = cut(i + 1) - lo;
+                if (!ni) continue;
+                const uint64_t tot = pk_tot[i * B2R_MAX_DEFS + d];
+                // row_start[lo + k] - base of the slice, k = 1 .. ni - 1, and the published total as k = ni: 8 bytes per string
+                if (ni > 1) CUDA_TRY(cudaMemcpyAsync(pk_rel[d] + lo, dpk.row_start[d] + lo + i + 1, (ni - 1) * 8, cudaMemcpyDeviceToHost, c->out_stream));
+                pk_rel[d][lo + ni - 1] = tot;
+                d2h += ni * 8;
+                if (dpk.entries[d] && run < pk->capacity) {
+                    uint64_t stored = tot;
+                    if (run + tot > pk->capacity) {                       // the one slice the capacity cuts: its offsets decide
+                        CUDA_TRY(cudaStreamSynchronize(c->out_stream));
+                        stored = pk_stored(run, pk->capacity, pk_rel[d] + lo, ni);
+                    }
+                    if (stored) {
+                        CUDA_TRY(cudaMemcpyAsync(pk->entries[d] + run, dpk.entries[d] + lo * pkw, stored * sizeof(b2r_row_count), cudaMemcpyDeviceToHost, c->out_stream));
+                        d2h += stored * sizeof(b2r_row_count);
+                    }
+                }
+                run += tot;
+            }
+        }
+    }
     for (const Copy& cp : copies)
         if (cp.stride && !cp.pinned && !cp.sparse && n) { CUDA_TRY(cudaMemcpyAsync(cp.host, cb + cp.off, n * cp.stride, cudaMemcpyDeviceToHost, c->out_stream)); d2h += n * cp.stride; }
     for (const Copy& cp : copies)
@@ -754,6 +927,22 @@ int host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, 
     if (trace) CUDA_TRY(cudaEventRecord(tev[3], c->out_stream));
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaStreamSynchronize(c->out_stream));
+    if (want_pk) {                                                        // row_start = the base of the slice + its relative offsets
+        if (!c->pool) c->pool.reset(new HostPool(c->opt.host_threads > 0 ? (unsigned)c->opt.host_threads : default_host_threads()));
+        for (uint32_t d = 0; d < c->n_defs; d++) {
+            if (!dpk.row_start[d]) continue;
+            uint64_t b = pk_base[d];
+            for (int i = 0; i < n_slices; i++) {
+                const uint64_t lo = cut(i), ni = cut(i + 1) - lo;
+                uint64_t* out = pk->row_start[d] + lo;
+                const uint64_t* rel = pk_rel[d] + lo;
+                c->pool->submit([out, rel, ni, b] { for (uint64_t k = 0; k < ni; k++) out[k] = b + (k ? rel[k - 1] : 0); });
+                if (ni) b += rel[ni - 1];
+            }
+            if (!hook || hook->last) pk->row_start[d][n] = b;
+        }
+        c->pool->wait();
+    }
     if (trace) {
         float h2d_end = 0, d2h_begin = 0, d2h_end = 0;
         cudaEventElapsedTime(&h2d_end, tev[0], tev[1]); cudaEventElapsedTime(&d2h_begin, tev[0], tev[2]); cudaEventElapsedTime(&d2h_end, tev[0], tev[3]);
@@ -820,7 +1009,7 @@ int multi_set_option(MultiState* m, const char* name, const char* value) {
 namespace {
 
 int multi_host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho, b2r_batch_status* result,
-                     const b2r_string_mult_outputs* sm = nullptr) {
+                     const b2r_string_mult_outputs* sm = nullptr, const b2r_string_mult_packed_outputs* pk = nullptr) {
     MultiState* m = c->multi;
     const int nd = (int)m->kids.size();
     if (!ho || (n && !h_offsets)) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
@@ -843,6 +1032,7 @@ int multi_host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_b
     std::vector<b2r_batch_status> res(nd);
     std::vector<std::string> errs(nd);
     std::vector<std::thread> threads;
+    PkChain chain(nd);                                                    // packed counts: device k's entries follow those of devices < k
     for (int k = 0; k < nd; k++)
         threads.emplace_back([&, k] {
             b2r_config* kid = m->kids[k];
@@ -869,11 +1059,20 @@ int multi_host_batch(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_b
                     if (s.endpoint_counts[d]) s.endpoint_counts[d] += lo * 2 * kid->packed[d].erows.size();
                 }
             }
+            b2r_string_mult_packed_outputs q{};                          // the entries' offset is known once devices < k have published
+            if (pk) {
+                q = *pk;
+                for (uint32_t d = 0; d < kid->n_defs; d++) {
+                    if (q.row_start[d]) q.row_start[d] += lo;
+                    if (q.endpoint_counts[d]) q.endpoint_counts[d] += lo * 2 * kid->packed[d].erows.size();
+                }
+            }
             MultiHook hook;
             hook.comm = m->comms[k]; hook.all_reduce = m->all_reduce; hook.error_string = m->error_string; hook.first = k == 0;
+            hook.chain = pk ? &chain : nullptr; hook.index = k; hook.last = k == nd - 1;
             memset(&res[k], 0, sizeof res[k]);
             static const uint64_t zero_off[1] = {0};
-            rcs[k] = host_batch(kid, entry, h_bytes, n ? h_offsets + lo : zero_off, hi - lo, &o, &res[k], &hook, sm ? &s : nullptr);
+            rcs[k] = host_batch(kid, entry, h_bytes, n ? h_offsets + lo : zero_off, hi - lo, &o, &res[k], &hook, sm ? &s : nullptr, pk ? &q : nullptr);
             if (rcs[k]) errs[k] = get_error();
         });
     for (auto& t : threads) t.join();
@@ -966,6 +1165,18 @@ int host_batch_mult(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_by
     return host_batch(c, entry, h_bytes, h_offsets, n, ho, result, nullptr, sm);
 }
 
+int host_batch_mult_packed(b2r_config* c, const DeviceEntry& entry, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
+                           const b2r_string_mult_packed_outputs* pk, b2r_batch_status* result) {
+    // the arguments are checked first (the same answer on any handle), then the device
+    if (!c) { set_error("null config"); return B2R_ERR_INVALID_ARG; }
+    if (!ho || !pk) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
+    const int rc = check_string_mult_packed(c, pk);
+    if (rc) return rc;
+    if (!c->multi && c->device < 0) { set_error("this handle was created without a device (device = -1): no CPU fallback exists"); return B2R_ERR_CUDA; }
+    if (c->multi) return multi_host_batch(c, entry, h_bytes, h_offsets, n, ho, result, nullptr, pk);
+    return host_batch(c, entry, h_bytes, h_offsets, n, ho, result, nullptr, nullptr, pk);
+}
+
 }  // namespace
 
 extern "C" {
@@ -978,6 +1189,16 @@ int b2r_match_batch_host_mult(b2r_config* c, const uint8_t* h_bytes, const uint6
 int b2r_match_batch_chunked_host_mult(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
                                       const b2r_string_mult_outputs* sm, b2r_batch_status* result) {
     return host_batch_mult(c, CHUNKED_ENTRY, h_bytes, h_offsets, n, ho, sm, result);
+}
+
+int b2r_match_batch_host_mult_packed(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
+                                     const b2r_string_mult_packed_outputs* pk, b2r_batch_status* result) {
+    return host_batch_mult_packed(c, BATCH_ENTRY, h_bytes, h_offsets, n, ho, pk, result);
+}
+
+int b2r_match_batch_chunked_host_mult_packed(b2r_config* c, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n, const b2r_outputs* ho,
+                                             const b2r_string_mult_packed_outputs* pk, b2r_batch_status* result) {
+    return host_batch_mult_packed(c, CHUNKED_ENTRY, h_bytes, h_offsets, n, ho, pk, result);
 }
 
 int b2r_match_substrs(b2r_config* c, const uint8_t* characters, uint64_t len, const b2r_outputs* h_out, b2r_batch_status* result) {

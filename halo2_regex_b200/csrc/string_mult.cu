@@ -11,6 +11,10 @@
 //                               one segment is sorted by row in the warp (bitonic) and written out; a longer string adds its
 //                               distinct rows into a dense per-string workspace of u32 counters.
 //   string_mult_compact_kernel  one CTA per string of several segments: the workspace row counters -> ascending entries.
+//
+// Packed layout (b2r_string_mult_packed): the two kernels above write every list whole into a slot workspace, then per pass
+//   string_mult_scan_kernel     one CTA per def: exclusive prefix of the list lengths -> row_start, carried across passes in device memory
+//   string_mult_pack_kernel     one warp per string: a list that fits below the capacity moves from its slots to entries + row_start[j]
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -247,6 +251,80 @@ __global__ void __launch_bounds__(COMPACT_THREADS) string_mult_compact_kernel(co
     }
 }
 
+// ---- packed layout (b2r_string_mult_packed): count into slots, then scan the counts and pack the lists back to back -------------
+constexpr int SCAN_THREADS = 1024;
+constexpr int SCAN_ITEMS = 8;             // counts per thread and tile: 8192 strings per tile, 128 tiles for 2^20 strings
+constexpr int PACK_THREADS = 256;
+
+struct PkDef {
+    const uint32_t* counts;               // this pass's strings: distinct rows (string_mult_kernel's n_entries)
+    const b2r_row_count* slots;           // [np][slot_pitch], or NULL: offsets only
+    b2r_row_count* entries;               // the caller's packed area
+    uint64_t* row_start;                  // of the CALL's string 0: this pass writes [j0, j0 + np]
+};
+
+struct PkParams {
+    uint64_t np, j0, capacity, slot_pitch;
+    uint64_t* carry;                      // [n_defs] entries of the earlier passes (device memory: no host round trip between passes)
+    uint64_t* host_total;                 // [n_defs] pinned host memory, or NULL: the running total after this pass
+    uint32_t n_defs;
+    PkDef def[B2R_MAX_DEFS];
+};
+
+// one CTA per def: the exclusive prefix of the pass's counts in tiles of SCAN_THREADS * SCAN_ITEMS, carried across tiles in a
+// register and across passes in `carry`.  One CTA streams 2^20 counts in well under a millisecond, against tens of milliseconds
+// of counting before it: a multi-CTA scan would buy nothing worth its second kernel
+__global__ void __launch_bounds__(SCAN_THREADS) string_mult_scan_kernel(const __grid_constant__ PkParams p) {
+    __shared__ uint64_t s_warp[SCAN_THREADS / 32];
+    const PkDef& f = p.def[blockIdx.x];
+    if (!f.row_start) return;
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint64_t carry = p.carry[blockIdx.x];
+    uint64_t* const out = f.row_start + p.j0;
+    constexpr uint64_t TILE = (uint64_t)SCAN_THREADS * SCAN_ITEMS;
+    for (uint64_t t0 = 0; t0 < p.np; t0 += TILE) {
+        const uint64_t first = t0 + (uint64_t)threadIdx.x * SCAN_ITEMS;
+        uint32_t v[SCAN_ITEMS];
+        uint64_t mine = 0;
+#pragma unroll
+        for (int k = 0; k < SCAN_ITEMS; k++) { v[k] = first + k < p.np ? f.counts[first + k] : 0u; mine += v[k]; }
+        uint64_t incl = mine;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const uint64_t x = __shfl_up_sync(0xFFFFFFFFu, incl, o); if (lane >= (uint32_t)o) incl += x; }
+        if (lane == 31) s_warp[warp] = incl;
+        __syncthreads();
+        uint64_t before = 0, tile = 0;
+        for (uint32_t w = 0; w < SCAN_THREADS / 32; w++) { const uint64_t x = s_warp[w]; if (w < warp) before += x; tile += x; }
+        uint64_t at = carry + before + incl - mine;
+#pragma unroll
+        for (int k = 0; k < SCAN_ITEMS; k++) { if (first + k < p.np) out[first + k] = at; at += v[k]; }
+        carry += tile;
+        __syncthreads();                                                  // s_warp is reused by the next tile
+    }
+    if (threadIdx.x == 0) {
+        out[p.np] = carry;                                                // the next pass overwrites it with the same value
+        p.carry[blockIdx.x] = carry;
+        if (p.host_total) p.host_total[blockIdx.x] = carry;
+    }
+}
+
+// one warp per (def, string): a list that fits whole below `capacity` moves from its slots to entries + row_start[j], 8 bytes a lane
+__global__ void __launch_bounds__(PACK_THREADS) string_mult_pack_kernel(const __grid_constant__ PkParams p) {
+    const uint32_t lane = threadIdx.x & 31;
+    const uint64_t n_units = p.np * p.n_defs;
+    for (uint64_t u = ((uint64_t)blockIdx.x * PACK_THREADS + threadIdx.x) >> 5; u < n_units; u += ((uint64_t)gridDim.x * PACK_THREADS) >> 5) {
+        const PkDef& f = p.def[u / p.np];
+        const uint64_t j = u % p.np;
+        if (!f.slots) continue;
+        const uint32_t cnt = f.counts[j];
+        const uint64_t start = f.row_start[p.j0 + j];
+        if (!cnt || start + cnt > p.capacity) continue;                  // no string is stored in part
+        const uint2* src = reinterpret_cast<const uint2*>(f.slots + j * p.slot_pitch);
+        uint2* dst = reinterpret_cast<uint2*>(f.entries + start);
+        for (uint32_t t = lane; t < cnt; t += 32) dst[t] = __ldcs(src + t);
+    }
+}
+
 }  // namespace
 
 bool string_mult_wanted(const b2r_config* c, const b2r_string_mult_outputs* sm, uint32_t d) {
@@ -343,6 +421,146 @@ int string_mult_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_of
     return B2R_OK;
 }
 
+// ---- packed layout ----------------------------------------------------------------------------------------------------------------
+bool string_mult_packed_wanted(const b2r_config* c, const b2r_string_mult_packed_outputs* pk, uint32_t d) {
+    return pk && d < c->n_defs && (pk->entries[d] || pk->row_start[d] || pk->endpoint_counts[d]);
+}
+
+int check_string_mult_packed(const b2r_config* c, const b2r_string_mult_packed_outputs* pk) {
+    if (!pk) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
+    for (uint32_t d = 0; d < c->n_defs; d++)
+        if (pk->entries[d] && !pk->row_start[d]) { set_error("def %u: entries without row_start", d); return B2R_ERR_INVALID_ARG; }
+    for (uint32_t d = 0; d < c->n_defs; d++)
+        if ((reinterpret_cast<uintptr_t>(pk->entries[d]) & 7) || (reinterpret_cast<uintptr_t>(pk->row_start[d]) & 7) ||
+            (reinterpret_cast<uintptr_t>(pk->endpoint_counts[d]) & 3)) {
+            set_error("def %u: entries and row_start must be 8-byte aligned, endpoint_counts 4-byte aligned", d);
+            return B2R_ERR_ALIGNMENT;
+        }
+    return B2R_OK;
+}
+
+namespace {
+
+// How a packed call over n strings runs: the counting kernels write each string's list into `pitch` = max_d min(M, T_d) slots
+// (never truncated) and its length into a u32, for `per_pass` strings at a time; scan and pack follow each pass
+struct PkShape {
+    bool scan = false;                    // some def wants offsets (else: endpoint counts only, one slot-less string_mult_impl call)
+    uint64_t pitch = 0, per_pass = 0, ws_bytes = 0;
+    size_t counts_off[B2R_MAX_DEFS] = {}, slots_off[B2R_MAX_DEFS] = {};
+};
+
+constexpr size_t PK_CARRY_BYTES = 256;    // [n_defs] u64 running totals at the front of ws_smpk
+
+PkShape pk_shape(const b2r_config* c, const b2r_string_mult_packed_outputs* pk, uint64_t n, uint64_t M) {
+    PkShape s;
+    uint64_t per_str = 0;
+    for (uint32_t d = 0; d < c->n_defs; d++) {
+        if (!pk->row_start[d]) continue;
+        s.scan = true;
+        per_str += 4;
+        if (pk->entries[d] && pk->capacity) s.pitch = std::max<uint64_t>(s.pitch, std::min<uint64_t>(M, c->packed[d].rows.size()));
+    }
+    if (!s.scan) return s;
+    for (uint32_t d = 0; d < c->n_defs; d++) if (pk->row_start[d] && pk->entries[d] && pk->capacity) per_str += s.pitch * 8;
+    const uint64_t cap = c->opt.chunked_max_maps > 0 ? (uint64_t)c->opt.chunked_max_maps : WS_CAP;
+    s.per_pass = std::max<uint64_t>(1, std::min<uint64_t>(n, cap / per_str));
+    size_t off = PK_CARRY_BYTES;
+    for (uint32_t d = 0; d < c->n_defs; d++) {
+        if (!pk->row_start[d]) continue;
+        s.counts_off[d] = off; off += align_up(s.per_pass * 4, 256);
+        if (pk->entries[d] && pk->capacity) { s.slots_off[d] = off; off += align_up(s.per_pass * s.pitch * 8, 256); }
+    }
+    s.ws_bytes = off;
+    return s;
+}
+
+// the slot-call outputs that a packed call hands to string_mult_impl (pointers into ws_smpk; endpoint counts: the caller's)
+b2r_string_mult_outputs pk_slot_outputs(const b2r_config* c, const b2r_string_mult_packed_outputs* pk, const PkShape& s, uint64_t j0) {
+    b2r_string_mult_outputs sm{};
+    sm.max_entries = (uint32_t)std::max<uint64_t>(1, s.pitch);
+    unsigned char* ws = (unsigned char*)c->ws_smpk.p;
+    for (uint32_t d = 0; d < c->n_defs; d++) {
+        if (pk->row_start[d]) sm.n_entries[d] = (uint32_t*)(ws + s.counts_off[d]);
+        if (pk->row_start[d] && pk->entries[d] && pk->capacity) sm.entries[d] = (b2r_row_count*)(ws + s.slots_off[d]);
+        if (pk->endpoint_counts[d]) sm.endpoint_counts[d] = pk->endpoint_counts[d] + j0 * 2 * c->packed[d].erows.size();
+    }
+    return sm;
+}
+
+}  // namespace
+
+int string_mult_packed_reserve(b2r_config* c, uint64_t n, uint64_t M, const b2r_string_mult_packed_outputs* pk) {
+    const PkShape s = pk_shape(c, pk, n, M);
+    int rc;
+    if (s.scan && (rc = c->ws_smpk.reserve(s.ws_bytes))) return rc;
+    // the per-string counters of strings longer than one segment, as string_mult_impl sizes them for a pass of per_pass strings
+    if (M - 1 > SEG) {
+        const b2r_string_mult_outputs sm = s.scan ? pk_slot_outputs(c, pk, s, 0) : b2r_string_mult_outputs{};
+        uint64_t per_str = 0;
+        for (uint32_t d = 0; d < c->n_defs; d++)
+            if (string_mult_wanted(c, &sm, d) || pk->endpoint_counts[d]) per_str += (c->packed[d].rows.size() + 2 * c->packed[d].erows.size()) * 4;
+        const uint64_t cap = c->opt.chunked_max_maps > 0 ? (uint64_t)c->opt.chunked_max_maps : WS_CAP;
+        const uint64_t m = s.scan ? s.per_pass : n;
+        if (per_str && (rc = c->ws_smult.reserve(std::min<uint64_t>(m, std::max<uint64_t>(1, cap / per_str)) * per_str))) return rc;
+    }
+    return B2R_OK;
+}
+
+int string_mult_packed_impl(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t M, void* const* states,
+                            uint64_t row_pitch, const b2r_string_status* status, const b2r_string_mult_packed_outputs* pk, uint64_t* host_total,
+                            cudaStream_t st, uint32_t* launches) {
+    bool any = false;
+    for (uint32_t d = 0; d < c->n_defs; d++) any = any || string_mult_packed_wanted(c, pk, d);
+    if (!any) return B2R_OK;
+    if (!n) {                                                             // row_start = {0}
+        for (uint32_t d = 0; d < c->n_defs; d++) if (pk->row_start[d]) CUDA_TRY(cudaMemsetAsync(pk->row_start[d], 0, 8, st));
+        if (host_total) for (uint32_t d = 0; d < c->n_defs; d++) host_total[d] = 0;
+        return B2R_OK;
+    }
+    const PkShape s = pk_shape(c, pk, n, M);
+    if (!s.scan) {                                                        // endpoint counts only: the slot call does it all
+        const b2r_string_mult_outputs sm = pk_slot_outputs(c, pk, s, 0);
+        return string_mult_impl(c, d_bytes, d_offsets, n, M, states, row_pitch, status, &sm, st, launches);
+    }
+    int rc;
+    if ((rc = string_mult_packed_reserve(c, n, M, pk))) return rc;
+    int n_sm = 0, max_smem = 0;
+    if ((rc = device_limits(&n_sm, &max_smem))) return rc;
+    unsigned char* const ws = (unsigned char*)c->ws_smpk.p;
+    PkParams p;
+    memset(&p, 0, sizeof p);
+    p.capacity = pk->capacity; p.slot_pitch = s.pitch; p.carry = (uint64_t*)ws; p.host_total = host_total; p.n_defs = c->n_defs;
+    bool pack = false;
+    for (uint32_t d = 0; d < c->n_defs; d++) {
+        PkDef& f = p.def[d];
+        if (!pk->row_start[d]) continue;
+        f.counts = (const uint32_t*)(ws + s.counts_off[d]);
+        f.row_start = pk->row_start[d];
+        if (pk->entries[d] && pk->capacity) { f.slots = (const b2r_row_count*)(ws + s.slots_off[d]); f.entries = pk->entries[d]; pack = true; }
+    }
+    CUDA_TRY(cudaMemsetAsync(p.carry, 0, c->n_defs * sizeof(uint64_t), st));
+    for (uint64_t j0 = 0; j0 < n; j0 += s.per_pass) {
+        const uint64_t np = std::min(s.per_pass, n - j0);
+        const b2r_string_mult_outputs sm = pk_slot_outputs(c, pk, s, j0);
+        void* sh[B2R_MAX_DEFS] = {};
+        for (uint32_t d = 0; d < c->n_defs; d++)
+            if (states[d]) sh[d] = (unsigned char*)states[d] + j0 * row_pitch * c->packed[d].state_width;
+        if ((rc = string_mult_impl(c, d_bytes, d_offsets + j0, np, M, sh, row_pitch, status + j0, &sm, st, launches))) return rc;
+        p.np = np; p.j0 = j0;
+        string_mult_scan_kernel<<<c->n_defs, SCAN_THREADS, 0, st>>>(p);
+        CUDA_TRY(cudaGetLastError());
+        (*launches)++;
+        if (pack) {
+            const uint64_t warps = np * c->n_defs;
+            const int grid = (int)std::min<uint64_t>((warps + PACK_THREADS / 32 - 1) / (PACK_THREADS / 32), (uint64_t)n_sm * 16);
+            string_mult_pack_kernel<<<grid, PACK_THREADS, 0, st>>>(p);
+            CUDA_TRY(cudaGetLastError());
+            (*launches)++;
+        }
+    }
+    return B2R_OK;
+}
+
 }  // namespace b2r
 
 using namespace b2r;
@@ -370,4 +588,29 @@ extern "C" int b2r_string_mult(b2r_config* c, const uint8_t* d_bytes, const uint
     if (!g.ok) { set_error("cudaSetDevice(%d) failed", c->device); return B2R_ERR_CUDA; }
     c->last_launches = 0;
     return string_mult_impl(c, d_bytes, d_offsets, n, M, o->states, o->row_pitch, o->status, sm, (cudaStream_t)cuda_stream, &c->last_launches);
+}
+
+extern "C" int b2r_string_mult_packed(b2r_config* c, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n, uint64_t total_bytes,
+                                      uint64_t max_chars_size, const b2r_outputs* o, const b2r_string_mult_packed_outputs* pk, void* cuda_stream) {
+    // the checks of b2r_string_mult, in the same order
+    if (!c) { set_error("null config"); return B2R_ERR_INVALID_ARG; }
+    if (!o || !pk || (n && !d_offsets) || (n && !d_bytes && total_bytes)) { set_error("null argument"); return B2R_ERR_INVALID_ARG; }
+    const uint64_t M = max_chars_size ? max_chars_size : c->max_chars;
+    if (M > 0xFFFFFFF0ull) { set_error("max_chars_size out of range"); return B2R_ERR_INVALID_ARG; }
+    int rc = check_string_mult_packed(c, pk);
+    if (rc) return rc;
+    bool any = false;
+    for (uint32_t d = 0; d < c->n_defs; d++) {
+        if (!string_mult_packed_wanted(c, pk, d)) continue;
+        any = true;
+        if (!o->states[d]) { set_error("def %u: per-string counts need the state column the match call wrote", d); return B2R_ERR_INVALID_ARG; }
+    }
+    if (any && !o->status) { set_error("per-string counts need the status column the match call wrote"); return B2R_ERR_INVALID_ARG; }
+    if ((rc = check_outputs(c, o, false, M))) return rc;
+    if (c->multi) { set_error("b2r_string_mult_packed takes device pointers of one device: a multi-device handle has no such call (use b2r_match_batch_host_mult_packed)"); return B2R_ERR_INVALID_ARG; }
+    if (c->device < 0) { set_error("this handle was created without a device (device = -1): no CPU fallback exists"); return B2R_ERR_CUDA; }
+    DeviceGuard g(c->device);
+    if (!g.ok) { set_error("cudaSetDevice(%d) failed", c->device); return B2R_ERR_CUDA; }
+    c->last_launches = 0;
+    return string_mult_packed_impl(c, d_bytes, d_offsets, n, M, o->states, o->row_pitch, o->status, pk, nullptr, (cudaStream_t)cuda_stream, &c->last_launches);
 }

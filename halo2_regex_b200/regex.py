@@ -204,6 +204,73 @@ class StringMultOutputs:
         return out
 
 
+class StringMultPacked:
+    """Per-string lookup multiplicities in the packed layout (include/b2r.h `b2r_string_mult_packed_outputs`) as torch tensors:
+    per def `entries[d]` (capacity, 2) int32 holding (row, count) pairs as u32, string j's list at
+    entries[d][row_start[d][j] : row_start[d][j + 1]]; `row_start[d]` (n + 1,) int64; `endpoint_counts[d]` (n, 2*E_d).
+    `capacity` defaults to the worst case n * max_d min(M, T_d), so every list is stored; a list is stored only when
+    row_start[d][j + 1] <= capacity.  `device`, `pin`, `fill`, `max_chars_size`: as for StringMultOutputs."""
+
+    WANT = ("entries", "row_start", "endpoint_counts")
+
+    def __init__(self, cfg, n, capacity=None, device=None, want=WANT, fill=None, pin=False, max_chars_size=None):
+        import torch
+        self.cfg, self.n = cfg, int(n)
+        self.m = int(max_chars_size) if max_chars_size else cfg.max_chars_size
+        self.capacity = int(capacity) if capacity is not None else self.n * max(min(self.m, t) for t in cfg.table_num_rows)
+        if device is None:
+            device = torch.device("cuda", cfg.device) if cfg.device >= 0 else "cpu"
+        dev = torch.device(device)
+        self.want = set(want)
+
+        def z(shape, dtype=torch.int32):
+            t = torch.empty(shape, dtype=dtype, device=dev, pin_memory=pin and dev.type == "cpu")
+            if fill is not None:
+                t.view(torch.uint8).fill_(fill)
+            return t
+
+        D = cfg.n_defs
+        self.entries = [z((self.capacity, 2)) if "entries" in self.want else None for _ in range(D)]
+        self.row_start = [z((self.n + 1,), torch.int64) if "row_start" in self.want or "entries" in self.want else None for _ in range(D)]
+        self.endpoint_counts = [z((self.n, 2 * cfg.endpoint_num_rows[d])) if "endpoint_counts" in self.want else None for d in range(D)]
+
+    def struct(self):
+        s = _abi.StringMultPackedStruct()
+        s.capacity = self.capacity
+        for d in range(self.cfg.n_defs):
+            for name in ("entries", "row_start", "endpoint_counts"):
+                t = getattr(self, name)[d]
+                getattr(s, name)[d] = None if t is None or t.numel() == 0 else t.data_ptr()
+        return s
+
+    def to_host(self):
+        """A copy of every buffer in host memory."""
+        h = StringMultPacked.__new__(StringMultPacked)
+        h.cfg, h.n, h.m, h.capacity, h.want = self.cfg, self.n, self.m, self.capacity, set(self.want)
+        for name in ("entries", "row_start", "endpoint_counts"):
+            setattr(h, name, [None if t is None else t.cpu() for t in getattr(self, name)])
+        return h
+
+    def stored(self, j, d):
+        """True when string j's list of def d is in `entries` (row_start[d][j + 1] <= capacity)."""
+        return self.entries[d] is not None and int(self.row_start[d][j + 1]) <= self.capacity
+
+    def entries_of(self, j, d):
+        """The (row, count) list of string j and def d as a (k, 2) uint32 array, rows ascending.  LookupError when it is not
+        stored (the capacity ran out before it)."""
+        if not self.stored(j, d):
+            raise LookupError(f"string {j}, def {d}: list not stored (row_start[{j + 1}] > capacity {self.capacity})")
+        a, b = int(self.row_start[d][j]), int(self.row_start[d][j + 1])
+        return self.entries[d][a:b].cpu().numpy().view(np.uint32)
+
+    def dense(self, j, d):
+        """The T_d-long count vector of string j (uint64): the mult[d] of a one-string batch of that string."""
+        out = np.zeros(self.cfg.table_num_rows[d], dtype=np.uint64)
+        e = self.entries_of(j, d)
+        out[e[:, 0]] = e[:, 1]
+        return out
+
+
 class RegexVerifyConfig:
     """reference src/lib.rs:97-113.  `configure` takes the two parameters that matter for witness generation
     (`max_chars_size`, `regex_defs`, src/lib.rs:126-131); `meta` / `gate` belong to the halo2 side and are ignored."""
@@ -328,6 +395,39 @@ class RegexVerifyConfig:
         call = lambda h, b, o, n_, st, res: fn(h, b, o, n_, st, C.byref(s), res)  # noqa: E731
         out, res = self._host_call(call, data, offsets, out, flags, check, sparse, reuse, kw)
         return out, sm, res
+
+    def match_batch_host_mult_packed(self, data, offsets, out=None, pk=None, flags=0, check=True, sparse=False, reuse=False, capacity=None, **kw):
+        """b2r_match_batch_host_mult_packed: match_batch_host plus the per-string lookup multiplicities in the packed layout
+        into `pk` (a host StringMultPacked, allocated here if not given).  Returns (out, pk, batch result)."""
+        return self._host_call_packed(lib.b2r_match_batch_host_mult_packed, data, offsets, out, pk, flags, check, sparse, reuse, capacity, kw)
+
+    def match_batch_chunked_host_mult_packed(self, data, offsets, out=None, pk=None, flags=0, check=True, sparse=False, reuse=False, capacity=None,
+                                             **kw):
+        """b2r_match_batch_chunked_host_mult_packed: match_batch_chunked_host plus the packed per-string lookup multiplicities."""
+        return self._host_call_packed(lib.b2r_match_batch_chunked_host_mult_packed, data, offsets, out, pk, flags, check, sparse, reuse, capacity, kw)
+
+    def _host_call_packed(self, fn, data, offsets, out, pk, flags, check, sparse, reuse, capacity, kw):
+        n = len(offsets) - 1
+        if pk is None:
+            pk = StringMultPacked(self, n, capacity=capacity, device="cpu")
+        s = pk.struct()
+        call = lambda h, b, o, n_, st, res: fn(h, b, o, n_, st, C.byref(s), res)  # noqa: E731
+        out, res = self._host_call(call, data, offsets, out, flags, check, sparse, reuse, kw)
+        return out, pk, res
+
+    def string_mult_packed_device(self, d_bytes, d_offsets, out, pk=None, max_chars_size=0, stream=None, capacity=None):
+        """b2r_string_mult_packed: string_mult_device's counts in the packed layout (StringMultPacked, on the device).
+        Asynchronous on `stream`.  Returns `pk`."""
+        import torch
+        if stream is None:
+            stream = torch.cuda.current_stream(d_bytes.device)
+        n = d_offsets.numel() - 1
+        if pk is None:
+            pk = StringMultPacked(self, n, capacity=capacity, device=d_bytes.device, max_chars_size=max_chars_size or None)
+        rc = lib.b2r_string_mult_packed(self._h, d_bytes.data_ptr(), d_offsets.data_ptr(), n, d_bytes.numel(), int(max_chars_size),
+                                        C.byref(out.struct()), C.byref(pk.struct()), stream.cuda_stream)
+        _raise(rc)
+        return pk
 
     def string_mult_device(self, d_bytes, d_offsets, out, sm=None, max_chars_size=0, stream=None, max_entries=None):
         """b2r_string_mult: per-string lookup multiplicities from the state columns and status that an earlier

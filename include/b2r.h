@@ -356,6 +356,47 @@ int b2r_match_batch_host_mult(b2r_config* cfg, const uint8_t* h_bytes, const uin
 int b2r_match_batch_chunked_host_mult(b2r_config* cfg, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n_strings,
                                       const b2r_outputs* h_out, const b2r_string_mult_outputs* h_sm, b2r_batch_status* result);
 
+/* ---- per-string lookup multiplicities, packed ---------------------------------------------------------------------------------------
+ * The same counts in a compressed-row layout: the lists of every string back to back, string j of def d at
+ * entries[d][row_start[d][j] .. row_start[d][j+1]).  No per-string cap to choose, and only the entries a string has are written
+ * (and, from the host entry points, copied back).
+ *
+ * Contract:
+ *   - Definition.  The list of string j and def d is exactly the list b2r_string_mult writes with max_entries >= min(M, T_d): rows
+ *     ascending, row 0 first with M - len.  A string flagged invalid or too long (or too long for the M passed) has an empty list,
+ *     row_start[j+1] == row_start[j], and all-zero endpoint counts.  endpoint_counts is that of b2r_string_mult_outputs.
+ *   - Offsets.  row_start[d] holds N + 1 u64, always complete: row_start[0] = 0, row_start[N] = the total, even when the total
+ *     exceeds capacity.
+ *   - Capacity.  The list of string j is stored only when row_start[j+1] <= capacity, so the stored lists are those of a prefix of
+ *     the strings, and no list is stored in part.  Every entry slot outside a stored list is left untouched.  entries[d] == NULL or
+ *     capacity == 0 writes the offsets only (a caller can size its buffer that way).
+ *   - Errors (nothing is enqueued): B2R_ERR_INVALID_ARG for entries[d] without row_start[d], and (device entry only) a NULL status
+ *     or NULL states[d] of a def whose counts are asked for, and a multi-device handle; B2R_ERR_ALIGNMENT for entries or row_start
+ *     not 8-byte aligned or endpoint_counts not 4-byte aligned; B2R_ERR_CUDA on a handle created with device = -1.
+ *   - Device entry.  Asynchronous on cuda_stream, no host synchronisation inside: once a first call of the same shape has sized the
+ *     workspace, the call can be captured in a CUDA graph.  The counting kernels of b2r_string_mult write each list whole into a
+ *     device workspace of max_d min(M, T_d) slots per string and def, in passes of at most 256 MiB of it (chunked_max_maps, when
+ *     set, bounds it instead; at least one string per pass), which the handle keeps; a scan and a pack kernel follow each pass.
+ *     b2r_last_launch_count counts the kernels of every pass: those of b2r_string_mult, one scan, and one pack when entries are
+ *     stored.
+ *   - Host entry points.  Every column, status, record and counter is what the call without _mult_packed writes (flags, pinned or
+ *     pageable buffers, NULL states / status, the small path, multi-device handles: as b2r_match_batch_host_mult).  No entry is
+ *     copied to the device; only the stored entries, row_start and the endpoint counts come back, and b2r_last_host_bytes reports
+ *     exactly those bytes on top of the call's own. */
+typedef struct b2r_string_mult_packed_outputs {
+    uint64_t capacity;                        /* entries reserved in entries[d] (per def) */
+    b2r_row_count* entries[B2R_MAX_DEFS];     /* string j: entries[d][row_start[d][j] .. row_start[d][j+1]), rows ascending; or NULL */
+    uint64_t* row_start[B2R_MAX_DEFS];        /* N + 1: exclusive prefix of the per-string list lengths, [N] = total; or NULL */
+    uint32_t* endpoint_counts[B2R_MAX_DEFS];  /* N * 2*E_d, dense, as in b2r_string_mult_outputs; or NULL */
+} b2r_string_mult_packed_outputs;
+
+int b2r_string_mult_packed(b2r_config* cfg, const uint8_t* d_bytes, const uint64_t* d_offsets, uint64_t n_strings, uint64_t total_bytes,
+                           uint64_t max_chars_size, const b2r_outputs* d_out, const b2r_string_mult_packed_outputs* d_pk, void* cuda_stream);
+int b2r_match_batch_host_mult_packed(b2r_config* cfg, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n_strings,
+                                     const b2r_outputs* h_out, const b2r_string_mult_packed_outputs* h_pk, b2r_batch_status* result);
+int b2r_match_batch_chunked_host_mult_packed(b2r_config* cfg, const uint8_t* h_bytes, const uint64_t* h_offsets, uint64_t n_strings,
+                                             const b2r_outputs* h_out, const b2r_string_mult_packed_outputs* h_pk, b2r_batch_status* result);
+
 /* ---- the step after the path: witness columns as field elements (SURVEY 8(f) rank 1) ------------------------------------------
  * The reference places every value of the path in a cell as Value::known(F::from(x as u64)) (src/lib.rs:342-347, 388-418), with
  * F = halo2curves::bn256::Fr in its own circuits (src/lib.rs:896).  b2r_column_to_fr converts a whole DEVICE column into an array

@@ -9,6 +9,7 @@
 //   AssignedRegexResult                                          reference src/lib.rs:79-93 (integer values, not cells)
 // Where the reference panics, these throw (std::runtime_error with the reference's panic text for an invalid transition).
 #pragma once
+#include <algorithm>
 #include <array>
 #include <cstdint>
 #include <memory>
@@ -214,6 +215,40 @@ public:
         if (rc == B2R_ERR_INVALID_TRANSITION) throw InvalidTransition(res);
         detail::check(rc);
         return w;
+    }
+
+    // The lookup multiplicities of every string of a batch, one list per string and def (b2r_match_batch_host_mult_packed): string
+    // j's (row, count) pairs of def d are entries[d][row_start[d][j] .. row_start[d][j+1]), rows ascending, row 0 first;
+    // endpoint_counts[d] holds 2*E_d counts per string.  chunked: b2r_match_batch_chunked_host_mult_packed.
+    struct StringMult {
+        std::vector<std::vector<b2r_row_count>> entries;
+        std::vector<std::vector<uint64_t>> row_start;
+        std::vector<std::vector<uint32_t>> endpoint_counts;
+    };
+    StringMult string_mult(const std::vector<std::vector<uint8_t>>& strings, bool chunked = false) const {
+        const size_t M = max_chars_size, D = regex_defs.size(), n = strings.size();
+        std::vector<uint8_t> bytes;
+        std::vector<uint64_t> offsets(n + 1, 0);
+        for (size_t j = 0; j < n; j++) { bytes.insert(bytes.end(), strings[j].begin(), strings[j].end()); offsets[j + 1] = bytes.size(); }
+        b2r_outputs out{};
+        out.row_pitch = (M + 31) & ~size_t(31); out.bitmap_pitch = ((M + 7) / 8 + 31) & ~size_t(31);
+        size_t pitch = 1;                                                 // no list is longer than min(M, T_d)
+        for (size_t d = 0; d < D; d++) pitch = std::max<size_t>(pitch, std::min<size_t>(M, b2r_table_num_rows(h_.get(), (uint32_t)d)));
+        StringMult s;
+        s.entries.resize(D); s.row_start.resize(D); s.endpoint_counts.resize(D);
+        b2r_string_mult_packed_outputs pk{};
+        pk.capacity = n * pitch;
+        for (size_t d = 0; d < D; d++) {
+            s.entries[d].resize(n * pitch); s.row_start[d].resize(n + 1); s.endpoint_counts[d].resize(n * 2 * b2r_endpoint_num_rows(h_.get(), (uint32_t)d));
+            pk.entries[d] = s.entries[d].data(); pk.row_start[d] = s.row_start[d].data(); pk.endpoint_counts[d] = s.endpoint_counts[d].data();
+        }
+        b2r_batch_status res{};
+        const int rc = (chunked ? b2r_match_batch_chunked_host_mult_packed : b2r_match_batch_host_mult_packed)(h_.get(), bytes.data(), offsets.data(), n,
+                                                                                                             &out, &pk, &res);
+        if (rc == B2R_ERR_INVALID_TRANSITION) throw InvalidTransition(res);
+        detail::check(rc);
+        for (size_t d = 0; d < D; d++) s.entries[d].resize(s.row_start[d][n]);
+        return s;
     }
 
     // match_substrs (src/lib.rs:311-315): one &[u8] in, the assigned values out

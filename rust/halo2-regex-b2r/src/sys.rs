@@ -54,6 +54,12 @@ pub struct b2r_string_mult_outputs {
     pub entries: [*mut b2r_row_count; B2R_MAX_DEFS], pub n_entries: [*mut u32; B2R_MAX_DEFS],
     pub endpoint_counts: [*mut u32; B2R_MAX_DEFS],
 }
+#[repr(C)]
+pub struct b2r_string_mult_packed_outputs {
+    pub capacity: u64,
+    pub entries: [*mut b2r_row_count; B2R_MAX_DEFS], pub row_start: [*mut u64; B2R_MAX_DEFS],
+    pub endpoint_counts: [*mut u32; B2R_MAX_DEFS],
+}
 
 extern "C" {
     pub fn b2r_last_error() -> *const c_char;
@@ -96,6 +102,12 @@ extern "C" {
                                      sm: *const b2r_string_mult_outputs, result: *mut b2r_batch_status) -> c_int;
     pub fn b2r_match_batch_chunked_host_mult(c: *mut b2r_config, bytes: *const u8, offsets: *const u64, n: u64, out: *const b2r_outputs,
                                              sm: *const b2r_string_mult_outputs, result: *mut b2r_batch_status) -> c_int;
+    pub fn b2r_string_mult_packed(c: *mut b2r_config, d_bytes: *const u8, d_offsets: *const u64, n: u64, total_bytes: u64, max_chars_size: u64,
+                                  d_out: *const b2r_outputs, d_pk: *const b2r_string_mult_packed_outputs, cuda_stream: *mut c_void) -> c_int;
+    pub fn b2r_match_batch_host_mult_packed(c: *mut b2r_config, bytes: *const u8, offsets: *const u64, n: u64, out: *const b2r_outputs,
+                                            pk: *const b2r_string_mult_packed_outputs, result: *mut b2r_batch_status) -> c_int;
+    pub fn b2r_match_batch_chunked_host_mult_packed(c: *mut b2r_config, bytes: *const u8, offsets: *const u64, n: u64, out: *const b2r_outputs,
+                                                    pk: *const b2r_string_mult_packed_outputs, result: *mut b2r_batch_status) -> c_int;
     pub fn b2r_batch_result(c: *mut b2r_config, cuda_stream: *mut c_void, out: *mut b2r_batch_status) -> c_int;
     pub fn b2r_column_to_fr(c: *mut b2r_config, d_col: *const c_void, kind: u32, d_offsets: *const u64, n_strings: u64, rows: u64,
                             pitch: u64, d_fr: *mut u64, cuda_stream: *mut c_void) -> c_int;
